@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the dense-flow hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one rank's batch of synthetic input: the 288-frame, 1500 x 2500
 GOES-CONUS-shaped brightness-temperature day of BASELINE.json configs[1] — forward+backward Farneback flow for
@@ -22,6 +22,13 @@ is 288*N frames, time-sharded one day per rank with NCCL point-to-point halo exc
 
 ``--impl reference`` times only that CPU implementation, with all host cores (a process pool over independent
 frames of work), and prints the same JSON line with "impl": "reference".
+
+``--dump-outputs DIR`` writes what the last timed step returned (rank 0's shard with N GPUs) to ``DIR/<name>.npy``:
+``forward_flow``, ``backward_flow``, ``diff``, ``convolve`` in float32 and ``sobel`` in float64.  An array of more than
+2**20 elements is stored as the 2**20 elements at fixed, seeded flat positions (sorted).  The operator results are NaN
+where an input pixel is NaN or a tap falls outside the series; such elements are written as 0 in ``<name>.npy`` and as 1
+in ``<name>_nan.npy`` (0 elsewhere, same dtype and shape), so every file is finite.  The files (48 MiB at most) of two
+builds run with the same arguments can be compared element for element: the synthetic input is seeded.
 """
 import argparse
 import gc
@@ -73,7 +80,13 @@ def parse_args():
     ap.add_argument("--no-detection", action="store_true", help="skip the detect_growth_markers extra (not the metric)")
     ap.add_argument("--detection-frames", type=int, default=48)
     ap.add_argument("--ref-workers", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (sampled when large)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; --impl reference has none")
     cfg = CONFIGS[a.config]
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if a.frames is None:
@@ -116,6 +129,25 @@ def measured_peak():
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_ELEMENTS = 1 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each device tensor to out_dir/<name>.npy: whole when it has at most DUMP_ELEMENTS elements, otherwise the
+    DUMP_ELEMENTS elements at flat positions drawn without replacement by a generator seeded with 0.  NaN elements are
+    written as 0 there and marked with 1 in out_dir/<name>_nan.npy."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        if t.numel() > DUMP_ELEMENTS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_ELEMENTS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy()
+        nan = np.isnan(a)
+        np.save(os.path.join(out_dir, name + ".npy"), np.where(nan, a.dtype.type(0), a))
+        np.save(os.path.join(out_dir, name + "_nan.npy"), nan.astype(a.dtype))
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -456,7 +488,7 @@ def run_b200(args):
     sampler.mark_begin()
     e0.record()
     for _ in range(args.steps):
-        step()
+        fl = step()
     e1.record()
     barrier()
     sampler.mark_end()
@@ -471,6 +503,10 @@ def run_b200(args):
         elapsed_ms = float(t.item())
     ms_per_step = elapsed_ms / args.steps
     value = T * world / (ms_per_step / 1e3)
+    if args.dump_outputs and rank == 0:
+        # before the strong-scaling run below reuses the buffers
+        dump_outputs(args.dump_outputs, {"forward_flow": fl.fwd, "backward_flow": fl.bwd, "diff": out_diff,
+                                         "sobel": out_sobel, "convolve": out_conv})
 
     # ---- multi-GPU evidence: the sharded result equals a local unsharded recomputation at the shard edges; the same
     # day split over the ranks (strong scaling) ------------------------------------------------------------------------

@@ -10,6 +10,7 @@ from oracle import detection_ops as det
 from oracle import flow_ops as ops
 
 import make_golden as mg
+import make_golden_reference_checks as rc
 
 BACKEND = "cv2" if ops.have_cv2() else "numpy"
 
@@ -131,12 +132,17 @@ def test_link_groups_random_graph():
             assert np.array_equal(got, want), (trial, overlap, absolute)
 
 
-def test_growth_rate_and_anvil_markers_against_the_unmodified_reference(multi):
-    """Build container only (skipped where /root/reference is absent): the oracle's get_growth_rate and
-    get_anvil_markers against the reference's own functions run under the dependency stubs."""
+def test_growth_rate_and_anvil_markers_against_the_unmodified_reference(multi, golden):
+    """The oracle's get_growth_rate and get_anvil_markers against stored results that match the reference's
+    (reference_checks.npz) and, where the reference is installed, against its own functions run under the dependency
+    stubs."""
+    g, wvd, fwd, bwd, r = multi
+    stored = golden("reference_checks")
+    for name, got in rc.growth_rate_and_anvil(wvd, fwd, bwd).items():
+        rc.assert_matches(stored, name, got)
     import refshim
     if not refshim.reference_available():
-        pytest.skip("reference not available")
+        return
     import sys
     import pandas as pd
     saved_path, saved_modules = list(sys.path), set(sys.modules)
@@ -144,7 +150,6 @@ def test_growth_rate_and_anvil_markers_against_the_unmodified_reference(multi):
         refshim.load_reference()
         from tobac_flow.flow import Flow
         from tobac_flow import detection
-        g, wvd, fwd, bwd, r = multi
         fl = Flow(fwd, bwd)
         t = pd.date_range("2020-01-01", periods=wvd.shape[0], freq="5min")
         da = refshim.DataArray(wvd, coords={"t": t}, dims=("t", "y", "x"), t=t)
@@ -153,7 +158,7 @@ def test_growth_rate_and_anvil_markers_against_the_unmodified_reference(multi):
             assert np.array_equal(detection.get_growth_rate(fl, da, method=m),
                                   det.get_growth_rate(wvd, dt, fwd, bwd, method=m, backend="cv2"), equal_nan=True)
         anvil = getattr(detection.get_anvil_markers, "__wrapped__", detection.get_anvil_markers)
-        for kw in (dict(), dict(threshold=-12, overlap=0.2, absolute_overlap=1, min_length=1)):
+        for kw in rc.ANVIL_KW:
             assert np.array_equal(np.asarray(anvil(fl, wvd, **kw)),
                                   det.get_anvil_markers(wvd, fwd, bwd, backend="cv2", **kw))
     finally:
@@ -166,17 +171,19 @@ def test_growth_rate_and_anvil_markers_against_the_unmodified_reference(multi):
         refshim._loaded = None
 
 
-def _bt_companion(wvd):
-    """A window brightness temperature that cools where the water-vapour difference grows (monotone map + offset)."""
-    return (250.0 - 2.2 * (wvd + 25.0)).astype(np.float32)
-
-
-def test_multichannel_markers_and_nan_gaussian_against_the_unmodified_reference(multi):
-    """Build container only: the oracle's detect_growth_markers_multichannel, its legacy multi-mask label filter and
-    nan_gaussian_filter against the reference's own functions run under the dependency stubs."""
+def test_multichannel_markers_and_nan_gaussian_against_the_unmodified_reference(multi, golden):
+    """The oracle's detect_growth_markers_multichannel, its legacy multi-mask label filter and nan_gaussian_filter
+    against stored results that match the reference's (reference_checks.npz) and, where the reference is installed,
+    against its own functions run under the dependency stubs."""
+    g, wvd, fwd, bwd, r = multi
+    stored = golden("reference_checks")
+    mine = rc.multichannel_and_nan_gaussian(wvd, fwd, bwd)
+    for name, a in mine.items():
+        rc.assert_matches(stored, name, a)
+    assert mine["multichannel_0_2"].max() >= 1 and mine["multichannel_1_2"].max() >= 1
     import refshim
     if not refshim.reference_available():
-        pytest.skip("reference not available")
+        return
     import sys
     import pandas as pd
     saved_path, saved_modules = list(sys.path), set(sys.modules)
@@ -184,28 +191,24 @@ def test_multichannel_markers_and_nan_gaussian_against_the_unmodified_reference(
         refshim.load_reference()
         from tobac_flow.flow import Flow
         from tobac_flow import detection
-        g, wvd, fwd, bwd, r = multi
-        bt = _bt_companion(wvd)
+        bt = rc.bt_companion(wvd)
         fl = Flow(fwd, bwd)
         t = pd.date_range("2020-01-01", periods=wvd.shape[0], freq="5min")
         da_w = refshim.DataArray(wvd, coords={"t": t}, dims=("t", "y", "x"), t=t)
         da_b = refshim.DataArray(bt, coords={"t": t}, dims=("t", "y", "x"), t=t)
         dt = np.full(wvd.shape[0], 5.0)
-        for kw in (dict(), dict(overlap=0.2, min_length=2, lower_threshold=0.2, upper_threshold=0.4)):
+        for kw in rc.MULTICHANNEL_KW:
             want = detection.detect_growth_markers_multichannel(fl, da_w, da_b, **kw)
             got = det.detect_growth_markers_multichannel(wvd, bt, dt, dt, fwd, bwd, backend="cv2", **kw)
             for a, b in zip(want, got):
                 a = np.asarray(a.data if hasattr(a, "data") and not isinstance(a, np.ndarray) else a)
                 assert np.array_equal(a, b, equal_nan=True)
             assert got[2].max() >= 1
-        x = wvd[:3].copy()
-        x[0, 10:14, 20:30] = np.nan
-        x[1, :, 50] = np.nan
-        x[2] = np.nan
-        for args in (((0, 2, 2),), ((0, 1.5, 1.5),)):
-            assert np.array_equal(detection.nan_gaussian_filter(x, *args), det.nan_gaussian_filter(x, *args), equal_nan=True)
-            assert np.array_equal(detection.nan_gaussian_filter(x, *args, propagate_nan=False),
-                                  det.nan_gaussian_filter(x, *args, propagate_nan=False), equal_nan=True)
+        x = rc.nan_gaussian_input(wvd)
+        for sigma in rc.GAUSS_SIGMAS:
+            assert np.array_equal(detection.nan_gaussian_filter(x, sigma), det.nan_gaussian_filter(x, sigma), equal_nan=True)
+            assert np.array_equal(detection.nan_gaussian_filter(x, sigma, propagate_nan=False),
+                                  det.nan_gaussian_filter(x, sigma, propagate_nan=False), equal_nan=True)
     finally:
         sys.path[:] = saved_path
         for name in set(sys.modules) - saved_modules:

@@ -121,24 +121,24 @@ def test_error_conventions():
         ops.convolve(d, z, z, method="bogus")
 
 
-def test_float64_and_integer_normalisation_against_the_unmodified_reference():
-    """Build container only: the oracle's pair quantisation for float64 / integer frames (numpy keeps float64 and
-    promotes integers, so the reference normalises in float64) against the reference's own to_8bit(linear_norm(.))."""
+def test_float64_and_integer_normalisation_against_the_unmodified_reference(golden):
+    """The oracle's pair quantisation for float64 / integer frames (numpy keeps float64 and promotes integers, so the
+    reference normalises in float64) against stored results that match the reference's (reference_checks.npz) and,
+    where the reference is installed, against its own to_8bit(linear_norm(.))."""
     import sys
     import refshim
-    import pytest
+    import make_golden_reference_checks as rc
+    stored = golden("reference_checks")
+    for name, got in rc.pair_quantisation().items():
+        rc.assert_matches(stored, name, got)
     if not refshim.reference_available():
-        pytest.skip("reference not available")
+        return
     from oracle import flow_ops as ops
-    from tobac_flow_b200 import synthetic
     saved_path, saved_modules = list(sys.path), set(sys.modules)
     try:
         refshim.load_reference()
         from tobac_flow.utils import to_8bit, linear_norm
-        bt = synthetic.bt_sequence(3, 120, 160, seed=3, nans=True).astype(np.float64) * 1.0000001
-        bt[1, 5:8] = np.nan
-        bi = np.nan_to_num(bt * 10).astype(np.int32)
-        for stack in (bt[0:2], bt[1:3], bi[0:2]):
+        for stack in rc.quantisation_stacks():
             r = to_8bit(linear_norm(stack), 0, 1)
             o = ops.pair_to_u8(stack[0], stack[1])
             assert np.array_equal(r[0], o[0]) and np.array_equal(r[1], o[1])

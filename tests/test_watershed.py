@@ -1,6 +1,6 @@
 """Semi-Lagrangian watershed: the native flood (tf_watershed_flood_host, a HOST function of the C-ABI library) and the
-oracle restatement against golden vectors produced by the reference's own Cython flood, and -- where that compiled
-reference is present (oracle/_ref, build container only) -- against it directly on random inputs.
+oracle restatement against golden vectors produced by the reference's own Cython flood, the native flood against stored
+labels on random inputs, and -- where that compiled reference is present (oracle/_ref) -- against it directly on them.
 
 The GPU-marked test runs the public ``Flow.watershed`` (device-side offset preparation + native flood).
 """
@@ -14,6 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 
 from oracle import build_ref_watershed, watershed_np  # noqa: E402
+import make_golden_reference_checks as rc  # noqa: E402
 import make_golden_watershed as mgw  # noqa: E402
 
 
@@ -32,12 +33,17 @@ def test_flood_matches_reference_golden(golden, name):
     assert np.array_equal(got_native, want)
 
 
-def test_flood_matches_compiled_reference_random():
+def test_flood_matches_compiled_reference_random(golden):
+    """The native flood against stored labels that match the reference's on random inputs (reference_checks.npz) and,
+    where the reference's Cython flood has been compiled (oracle/_ref), against it directly."""
+    stored = golden("reference_checks")
+    for name, got in rc.watershed_random(flood=native_flood).items():
+        rc.assert_matches(stored, name, got)
     ref = build_ref_watershed.load()
     if ref is None:
-        pytest.skip("oracle/_ref/_ref_watershed not built (python oracle/build_ref_watershed.py; build container only)")
-    for seed in range(6):
-        c = mgw.case(100 + seed, T=4, H=24 + seed, W=31, conn=1 + seed % 2, ties=bool(seed % 2))
+        return
+    for seed in rc.WATERSHED_SEEDS:
+        c = rc.watershed_case(seed)
         a = watershed_np.watershed(c["fwd"], c["bwd"], c["field"], c["markers"], c["mask"], c["conn"],
                                    flood=lambda *x: ref.watershed_raveled(x[0], x[1], x[2], x[3], x[4], x[5], x[6], x[7],
                                                                           np.zeros(3, np.int32), 0.0, x[8], False))
