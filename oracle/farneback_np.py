@@ -231,18 +231,29 @@ def poly_exp(img: np.ndarray, n: int = 5, sigma: float = 1.1) -> np.ndarray:
 # ----------------------------------------------------------------------------------------------
 # FarnebackUpdateMatrices
 # ----------------------------------------------------------------------------------------------
+def _border_band(n: int) -> np.ndarray:
+    """OpenCV's test ``(unsigned)(x - BORDER) >= (unsigned)(n - BORDER*2)`` along one axis.  For n >= 10 it selects the
+    five indices next to either edge.  For n < 10 the right-hand side wraps: it then selects only n - 5 <= x < 5, so on a
+    side of 6..9 px some indices within 5 px of an edge are not attenuated (unless the other axis selects the pixel)."""
+    i = np.arange(n, dtype=np.int64)
+    return ((i - 5) & 0xFFFFFFFF) >= ((n - 10) & 0xFFFFFFFF)
+
+
 def border_scale(h: int, w: int) -> np.ndarray:
-    sx = np.ones(w, dtype=F32)
-    sy = np.ones(h, dtype=F32)
-    for i in range(5):
-        if i < w:
-            sx[i] *= BORDER_ATTEN[i]
-            sx[w - 1 - i] *= BORDER_ATTEN[i]
-        if i < h:
-            sy[i] *= BORDER_ATTEN[i]
-            sy[h - 1 - i] *= BORDER_ATTEN[i]
-    # OpenCV multiplies (x<B ? b[x] : 1)*(x>=w-B ? b[w-x-1] : 1)*(y...)*(y...) left to right in fp32
-    return (sx[None, :] * sy[:, None]).astype(F32)
+    """The attenuation FarnebackUpdateMatrices applies to (r2..r6): 1 where neither axis' band test holds, else the
+    product (x<B ? b[x] : 1)*(x>=w-B ? b[w-x-1] : 1)*(y<B ? b[y] : 1)*(y>=h-B ? b[h-y-1] : 1), left to right in fp32."""
+    def factors(n):
+        lo = np.ones(n, dtype=F32)
+        hi = np.ones(n, dtype=F32)
+        for i in range(min(5, n)):
+            lo[i] = BORDER_ATTEN[i]
+            hi[n - 1 - i] = BORDER_ATTEN[i]
+        return lo, hi
+    xl, xr = factors(w)
+    yt, yb = factors(h)
+    prod = ((xl * xr)[None, :] * yt[:, None]).astype(F32) * yb[:, None]
+    band = _border_band(w)[None, :] | _border_band(h)[:, None]
+    return np.where(band, prod, F32(1)).astype(F32)
 
 
 def update_matrices(R0: np.ndarray, R1: np.ndarray, flow: np.ndarray) -> np.ndarray:

@@ -100,10 +100,23 @@ def test_flow_blob_known_answers(tfb, golden):
     assert np.array_equal(f.backward_flow[0], -f.forward_flow[0])
 
 
-@pytest.mark.parametrize("shape", [(10, 15), (33, 47), (64, 64), (100, 259), (257, 130)])
+# tiny frames: single rows / columns, frames narrower than the 6-column halo of a strip, sides of 6..9 px (OpenCV's
+# border band test wraps there), widths on either side of a 116-column strip boundary.  They take the analytic texture:
+# bt_sequence's field is noise low-passed at 12 px, and on a side of a few px only one Fourier mode of it is left, a
+# one-directional sinusoid on which the flow along the stripes is set by rounding (two float64 restatements of
+# OpenCV already differ by 0.1 px at 7 x 12).
+TINY_FRAMES = [(1, 1), (1, 40), (40, 1), (2, 3), (5, 5), (7, 12), (12, 7), (6, 40), (40, 9), (13, 13), (31, 33),
+               (64, 115), (64, 116), (64, 117), (40, 233)]
+
+
+@pytest.mark.parametrize("shape", [(10, 15), (33, 47), (64, 64), (100, 259), (257, 130)] + TINY_FRAMES)
 def test_flow_vs_oracle_odd_sizes(tfb, shape):
     h, w = shape
-    bt = synthetic.bt_sequence(3, h, w, seed=h * 7 + w, nans=False)
+    if shape in TINY_FRAMES:
+        motions = [synthetic.shift_motion(1.0, 2.0), synthetic.shift_motion(-2.0, 1.0)]
+        bt = synthetic.moving_texture(h, w, motions, seed=h * 7 + w)
+    else:
+        bt = synthetic.bt_sequence(3, h, w, seed=h * 7 + w, nans=False)
     f = tfb.create_flow(bt)
     ref_f, ref_b = ops.create_flow(bt, backend="cv2" if ops.have_cv2() else "numpy")
     assert_flow_close(f.forward_flow, ref_f, 2e-3, 2e-2)
@@ -498,7 +511,7 @@ def test_iteration_kernels_agree(tfb):
     from tobac_flow_b200 import _lib
     lib = _lib.load()
     try:
-        for shape in ((3, 100, 100), (3, 97, 131), (2, 150, 258), (2, 64, 1101)):
+        for shape in ((3, 100, 100), (3, 97, 131), (2, 150, 258), (2, 64, 1101), (3, 12, 7), (3, 40, 117)):
             bt = synthetic.bt_sequence(shape[0], shape[1], shape[2], seed=77 + shape[2], nans=True)
             res = {}
             for k in (0, 1, 3, 4, 5):

@@ -51,6 +51,34 @@ def test_farneback_matches_cv2(shape):
 
 
 @pytest.mark.skipif(not flow_ops.have_cv2(), reason="cv2 not importable")
+def test_farneback_matches_cv2_on_tiny_frames():
+    """Every side 1..15 against a side of 40, both ways round: one pyramid level, the box window and the polynomial
+    expansion wider than the frame, and OpenCV's border band test, which on sides of 6..9 px leaves some pixels
+    within 5 px of an edge unattenuated."""
+    import cv2
+    shapes = [(s, 40) for s in range(1, 16)] + [(40, s) for s in range(1, 16)] + [(7, 7), (6, 13)]
+    for h, w in shapes:
+        bt = synthetic.moving_texture(h, w, [synthetic.rotation_motion(2.0)], seed=h * 100 + w)
+        q0, q1 = flow_ops.pair_to_u8(bt[0], bt[1])
+        for a, b in ((q0, q1), (q1, q0)):
+            ref = cv2.FarnebackOpticalFlow_create().calc(a, b, None)
+            e = epe(fb.farneback(a, b), ref)
+            assert e.mean() < 1e-5 and e.max() < 1e-4, ((h, w), e.mean(), e.max())
+
+
+def test_border_scale_band_rule():
+    """FarnebackUpdateMatrices attenuates where (unsigned)(x - 5) >= (unsigned)(w - 10) or the same holds for y."""
+    s = fb.border_scale(40, 7)                    # w = 7: only columns 2..4 pass the x test
+    assert (s[20, 2:5] < 1).all() and s[20, 0] == 1 and s[20, 1] == 1 and s[20, 5] == 1 and s[20, 6] == 1
+    assert s[0, 0] == np.float32(np.float32(np.float32(0.14) * np.float32(1)) * np.float32(0.14))
+    s = fb.border_scale(3, 3)                     # every factor applies: ((x0 * x1) * y0) * y1 in fp32
+    f = [np.float32(v) for v in (0.14, 0.14, 0.4472)]
+    assert s[1, 1] == np.float32(np.float32(np.float32(f[1] * f[1]) * f[1]) * f[1])
+    s = fb.border_scale(20, 30)
+    assert (s[5:15, 5:25] == 1).all() and s[4, 10] == np.float32(0.4472) and s[10, 29] == np.float32(0.14)
+
+
+@pytest.mark.skipif(not flow_ops.have_cv2(), reason="cv2 not importable")
 def test_stages_match_cv2():
     import cv2
     img = (synthetic.base_field(200, 300, 3) * 255).astype(np.float32)

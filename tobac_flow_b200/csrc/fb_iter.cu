@@ -153,8 +153,8 @@ __device__ __forceinline__ void issue_taps_v3(TapsV3& t, const float4* __restric
 // FarnebackUpdateMatrices for one pixel: (A, B, C) = ((M0, M2), (M3, M4), M1); c / c4 = R0 at the pixel, f = its flow.
 // The (c0, c1) and (c2, c3) halves of every float4 tap are blended with packed FMAs: per lane exactly the chain of
 // blend4() (fb_iter_common.cuh), so the terms carry the same bits as the scalar kernel's.
-__device__ __forceinline__ void matrix_v3(const TapsV3& t, float4 c, float c4, float2 f, int y, int h, float sc_x, f2& mA,
-                                          f2& mB, float& mC) {
+__device__ __forceinline__ void matrix_v3(const TapsV3& t, float4 c, float c4, float2 f, int y, int h, float sc_x,
+                                          bool band_x, f2& mA, f2& mB, float& mC) {
     f2 r23, r45;
     float r6;
     const f2 half2 = make_float2(0.5f, 0.5f), minus1 = make_float2(-1.f, -1.f);
@@ -174,7 +174,7 @@ __device__ __forceinline__ void matrix_v3(const TapsV3& t, float4 c, float c4, f
     }
     r23 = mul2(fma2(r23, minus1, lo2(c)), half2);                // (c - r) * 0.5: the FMA with -1 is the exact subtraction
     float m[5];
-    terms_from_blend(r23.x, r23.y, r45.x, r45.y, r6, f.x, f.y, border_scale(sc_x, y, h), m);
+    terms_from_blend(r23.x, r23.y, r45.x, r45.y, r6, f.x, f.y, border_scale(sc_x, band_x, y, h), m);
     mA = make_float2(m[0], m[2]);
     mC = m[1];
     mB = make_float2(m[3], m[4]);
@@ -219,6 +219,7 @@ fb_iter_v3_kernel(const float* __restrict__ R, long long img_stride, const float
     const int gx = min(max(xs + tid, 0), w - 1);
     const int gxs = gx - cx0;
     const float sc_x = border_factor(gx, w);
+    const bool band_x = border_band(gx, w);
     const int hr = tid >> 5, cg = tid & 31;
     const unsigned skb0 = (unsigned)(reinterpret_cast<uintptr_t>(R0b) >> 2), skf0 = (unsigned)(reinterpret_cast<uintptr_t>(fin) >> 3);
 
@@ -347,10 +348,10 @@ fb_iter_v3_kernel(const float* __restrict__ R, long long img_stride, const float
             float mC;
             if (PF == 1) {
                 issue_taps_v3(S1, R1a, R1b, w, h, gx, row_y(i + 1), fnext);
-                matrix_v3(S0, c, c4, fcur, y_cur, h, sc_x, mA, mB, mC);
+                matrix_v3(S0, c, c4, fcur, y_cur, h, sc_x, band_x, mA, mB, mC);
             } else {
                 TapsV3& st = (j & 1) ? S1 : S0;
-                matrix_v3(st, c, c4, fcur, y_cur, h, sc_x, mA, mB, mC);
+                matrix_v3(st, c, c4, fcur, y_cur, h, sc_x, band_x, mA, mB, mC);
                 issue_taps_v3(st, R1a, R1b, w, h, gx, row_y(i + 2), fnext);
             }
             if (j == 0) { Pa = mA; Pb = mB; Pc = mC; }

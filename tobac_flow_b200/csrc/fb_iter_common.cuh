@@ -69,8 +69,19 @@ __device__ __forceinline__ void bilinear_weights(float fx, float fy, float& a00,
 __device__ __forceinline__ float blend4(float a00, float a01, float a10, float a11, float p00, float p01, float p10, float p11) {
     return fmaf(a11, p11, fmaf(a10, p10, fmaf(a01, p01, __fmul_rn(a00, p00))));
 }
-__device__ __forceinline__ float border_scale(float sc_x, int y, int h) {
-    return (sc_x != 1.f || (unsigned)(y - 5) >= (unsigned)(h - 10)) ? __fmul_rn(sc_x, border_factor(y, h)) : 1.f;
+// OpenCV's test for the attenuated band along one axis, (unsigned)(p - 5) >= (unsigned)(n - 10): p < 5 || p >= n - 5
+// when n >= 10.  For n < 10 the right-hand side wraps and only n - 5 <= p < 5 passes, so on a side of 6..9 px some
+// pixels within 5 px of an edge are left unattenuated unless the other axis selects them.
+__device__ __forceinline__ bool border_band(int p, int n) { return (unsigned)(p - 5) >= (unsigned)(n - 10); }
+// The scale of FarnebackUpdateMatrices: 1 unless either axis' band test holds, else the four edge factors multiplied
+// left to right in fp32; sc_x = border_factor(x, w) is the product of the first two.
+__device__ __forceinline__ float border_scale(float sc_x, bool band_x, int y, int h) {
+    if (!band_x && !border_band(y, h)) return 1.f;
+    float s = sc_x;
+    if (y < 5) s = __fmul_rn(s, y < 2 ? 0.14f : 0.4472f);
+    const int q = h - 1 - y;
+    if (q < 5) s = __fmul_rn(s, q < 2 ? 0.14f : 0.4472f);
+    return s;
 }
 
 // Chunk grid of the strip march: rows per chunk minimising (waves of resident CTAs) x (rows a CTA marches, including its

@@ -83,7 +83,7 @@ __device__ __forceinline__ void issue_taps(Taps& t, const RPlanes& R, int w, int
 }
 
 // FarnebackUpdateMatrices for one pixel from its loaded taps (explicit roundings: see fb_iter_common.cuh)
-__device__ __forceinline__ void matrix_from_taps(const Taps& t, int h, float sc_x, float m[5]) {
+__device__ __forceinline__ void matrix_from_taps(const Taps& t, int h, float sc_x, bool band_x, float m[5]) {
     float r2, r3, r4, r5, r6;
     if (t.inside) {
         float a00, a01, a10, a11;
@@ -104,7 +104,7 @@ __device__ __forceinline__ void matrix_from_taps(const Taps& t, int h, float sc_
     }
     r2 = __fmul_rn(__fsub_rn(t.c.x, r2), 0.5f);
     r3 = __fmul_rn(__fsub_rn(t.c.y, r3), 0.5f);
-    terms_from_blend(r2, r3, r4, r5, r6, t.dx, t.dy, border_scale(sc_x, t.y, h), m);
+    terms_from_blend(r2, r3, r4, r5, r6, t.dx, t.dy, border_scale(sc_x, band_x, t.y, h), m);
 }
 
 template <bool TM>
@@ -150,6 +150,7 @@ fb_iter_scalar_kernel(const float* __restrict__ R, long long img_stride, const f
     // M-phase identity: one column of the strip (replicate-clamped = the box filter's border rule)
     const int gx = min(max(x0 - IT_HALO + tid, 0), w - 1);
     const float sc_x = border_factor(gx, w);
+    const bool band_x = border_band(gx, w);
     // H-phase identity: a warp owns one row of the batch, a lane four adjacent outputs
     const int hr = tid >> 5, cg = tid & 31;
 
@@ -196,7 +197,7 @@ fb_iter_scalar_kernel(const float* __restrict__ R, long long img_stride, const f
             issue_taps(nxt, RP, w, h, gx, row_y(i + 1), fq[j]);
             fq[j] = ld_stream(fin + row_y(i + 5) * w + gx);
             float m[5];
-            matrix_from_taps(cur, h, sc_x, m);
+            matrix_from_taps(cur, h, sc_x, band_x, m);
             if constexpr (TM) {
                 float xold[5];
 #pragma unroll

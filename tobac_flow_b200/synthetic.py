@@ -6,6 +6,8 @@ G2  ``bt_sequence``  — brightness-temperature-like float32 ``(T, H, W)``: a sm
                        by (+1, +2) px/frame, a warm clear-sky plateau at 285 K, growing cold cores, and the
                        NaN patterns of ``tobac_flow/dataloader.py:288-357`` (bad pixels, a missing stripe,
                        a whole missing frame).
+G3  ``moving_texture`` — an analytic texture under prescribed, per-pair motion (shifts, rotation, zoom, a
+                       discontinuity), exact in every frame: flow tests against OpenCV beyond a constant roll.
 
 ``bt_sequence`` works on numpy (tests, CPU baseline) and on torch tensors (bench, on the GPU) from the
 same seeded base field, so the CPU baseline and the CUDA path see identical inputs.
@@ -115,6 +117,62 @@ def bt_sequence(T: int, H: int, W: int, seed: int = 1234, nans: bool = True, dev
     for t in range(T):
         out[t] = bt_frame(base_t, t, cores, plan, T)
     return out
+
+
+def texture(x, y, seed: int = 0):
+    """Analytic texture: 12 seeded sinusoids (wavelengths 10-45 px) around 250 K, float64 at arbitrary (x, y)."""
+    rng = np.random.default_rng(seed)
+    f = np.full(np.broadcast(x, y).shape, 250.0)
+    for _ in range(12):
+        k = 2.0 * np.pi / rng.uniform(10.0, 45.0)
+        th = rng.uniform(0.0, 2.0 * np.pi)
+        f += rng.uniform(1.5, 4.0) * np.sin(k * np.cos(th) * x + k * np.sin(th) * y + rng.uniform(0.0, 2.0 * np.pi))
+    return f
+
+
+# motions d(x, y, H, W) -> (u, v) for moving_texture: frame k + 1 at x shows frame k at x - d(x), so the forward flow
+# of the pair is ~ d
+def shift_motion(u: float, v: float):
+    return lambda x, y, H, W: (np.full_like(x, u), np.full_like(y, v))
+
+
+def rotation_motion(deg: float):
+    """Rotation by ``deg`` about the frame centre."""
+    def d(x, y, H, W):
+        cx, cy, a = (W - 1) / 2.0, (H - 1) / 2.0, np.deg2rad(deg)
+        rx = cx + np.cos(a) * (x - cx) + np.sin(a) * (y - cy)       # the point that rotates onto (x, y)
+        ry = cy - np.sin(a) * (x - cx) + np.cos(a) * (y - cy)
+        return x - rx, y - ry
+    return d
+
+
+def zoom_motion(factor: float):
+    """Magnification by ``factor`` about the frame centre (outward flow for factor > 1)."""
+    def d(x, y, H, W):
+        cx, cy = (W - 1) / 2.0, (H - 1) / 2.0
+        return (x - cx) * (1.0 - 1.0 / factor), (y - cy) * (1.0 - 1.0 / factor)
+    return d
+
+
+def split_motion(s: float):
+    """+s px along x left of the centre column, -s px right of it: a motion discontinuity."""
+    return lambda x, y, H, W: (np.where(x < (W - 1) / 2.0, s, -s), np.zeros_like(y))
+
+
+def moving_texture(H: int, W: int, motions, seed: int = 0) -> np.ndarray:
+    """(len(motions) + 1, H, W) float32 frames of ``texture``, each pair with its own motion.
+
+    Frame k is the texture at p_k(x), p_0 the identity and p_k(x) = p_{k-1}(x - d_k(x)), evaluated in float64: no frame
+    carries interpolation error."""
+    y, x = np.mgrid[0:H, 0:W].astype(np.float64)
+    frames = []
+    for k in range(len(motions) + 1):
+        px, py = x, y
+        for m in reversed(motions[:k]):
+            u, v = m(px, py, H, W)
+            px, py = px - u, py - v
+        frames.append(texture(px, py, seed))
+    return np.stack(frames).astype(np.float32)
 
 
 def wvd_from_bt(bt):
