@@ -158,6 +158,43 @@ int tf_variational_refinement(const uint8_t* q0, const uint8_t* q1, float* fwd, 
                               long long bwd_stride, int n_pairs, int H, int W, const tf_vr_params* p /* host */,
                               void* workspace, size_t workspace_bytes, void* stream);
 
+/* cv2.DISOpticalFlow parameters (patch size 8, mean normalisation and spatial propagation on: the presets' values and
+ * the only ones built).  tf_dis_default_params(p, preset) gives cv2.DISOpticalFlow_create(preset) for preset 0
+ * (ULTRAFAST), 1 (FAST, the factory default) and 2 (MEDIUM), with max_value = 0. */
+typedef struct tf_dis_params {
+    int finest_scale;                       /* 2 / 2 / 1 (a frame too small for it lowers it, as calc() does) */
+    int patch_stride;                       /* 4 / 4 / 3  (1..8) */
+    int gradient_descent_iterations;        /* 12 / 16 / 25 */
+    int variational_refinement_iterations;  /* 0 / 5 / 5  (fixed-point iterations of the per-scale refinement) */
+    float vr_alpha, vr_delta, vr_gamma;     /* 20, 5, 10 */
+    float vr_epsilon;                       /* 0.01 (the standalone refinement's default is 0.001) */
+    float max_value;                        /* clamp of the final flow (create_flow's +-max_value); <= 0 disables */
+} tf_dis_params;
+
+void tf_dis_default_params(tf_dis_params* p /* host */, int preset);
+
+/* HOST: the scales calc() runs for an H x W frame: *finest, *coarsest and, for finest <= s <= coarsest, the scale
+ * image size hs[s] x ws[s] (host arrays of >= 16 ints; any pointer may be NULL).  Fails (TF_ERR_INVALID_ARGUMENT)
+ * where OpenCV refuses the frame, and with TF_ERR_UNSUPPORTED where OpenCV would switch to patch size 12. */
+int tf_dis_scale_plan(int H, int W, const tf_dis_params* p /* host */, int* finest, int* coarsest, int* hs /* host */,
+                      int* ws /* host */);
+
+/* Bytes of scratch tf_dis_pairs needs for `n_pairs` pairs of H x W frames (0 for a frame the plan refuses). */
+size_t tf_dis_workspace_bytes(int n_pairs, int H, int W, const tf_dis_params* p /* host */);
+
+/*
+ * Forward and backward DIS flow of n_pairs quantised pairs: cv2.DISOpticalFlow.calc(q0, q1, None) and
+ * .calc(q1, q0, None) with a fresh object per call, plus the +-max_value clamp.  Addressing as tf_farneback_pairs.
+ */
+int tf_dis_pairs(const uint8_t* q0, const uint8_t* q1, float* fwd, long long fwd_stride, float* bwd, long long bwd_stride,
+                 int n_pairs, int H, int W, const tf_dis_params* p /* host */, void* workspace, size_t workspace_bytes,
+                 void* stream);
+
+/* Stage entry point: scale image `scale` of the DIS pyramid of each of the n_img u8 frames q (n_img, H, W) and its
+ * spatialGradient: img (n_img, hs, ws) u8, gx / gy (n_img, hs, ws) int16.  workspace: tf_dis_workspace_bytes(n_img, ..) */
+int tf_dis_scale_images(const uint8_t* q, int n_img, int H, int W, const tf_dis_params* p /* host */, int scale,
+                        uint8_t* img, int16_t* gx, int16_t* gy, void* workspace, size_t workspace_bytes, void* stream);
+
 /*
  * One smooth_flow_step (tobac_flow/flow.py:530-568) on n_pairs (fwd, bwd) fields in place semantics:
  * fwd' = nanmean(fwd, -warp(bwd by fwd)), bwd' = nanmean(bwd, -warp(fwd by bwd)), both from the old

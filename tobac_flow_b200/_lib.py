@@ -27,7 +27,8 @@ EXPORTS = (
     "tf_ccl_workspace_bytes", "tf_flat_label", "tf_binary_fill_holes", "tf_gaussian_filter_yx", "tf_curvature_mask",
     "tf_binary_opening_cross", "tf_grey_opening_cross", "tf_scale_frames", "tf_mask_multiply", "tf_threshold_ge",
     "tf_label_max", "tf_label_overlap_count", "tf_label_link_groups", "tf_relabel", "tf_label_stats",
-    "tf_watershed_flood_host",
+    "tf_watershed_flood_host", "tf_dis_default_params", "tf_dis_scale_plan", "tf_dis_workspace_bytes", "tf_dis_pairs",
+    "tf_dis_scale_images",
 )
 
 KERNEL_CLASSES = ("normalise", "pyramid", "polyexp", "flow_upsample", "fb_iter_coarse", "fb_iter_fullres",
@@ -47,6 +48,15 @@ class VrParams(ctypes.Structure):
         ("alpha", ctypes.c_float), ("delta", ctypes.c_float), ("gamma", ctypes.c_float), ("omega", ctypes.c_float),
         ("fixed_point_iterations", ctypes.c_int), ("sor_iterations", ctypes.c_int), ("zeta", ctypes.c_float),
         ("epsilon", ctypes.c_float),
+    ]
+
+
+class DisParams(ctypes.Structure):
+    _fields_ = [
+        ("finest_scale", ctypes.c_int), ("patch_stride", ctypes.c_int), ("gradient_descent_iterations", ctypes.c_int),
+        ("variational_refinement_iterations", ctypes.c_int), ("vr_alpha", ctypes.c_float),
+        ("vr_delta", ctypes.c_float), ("vr_gamma", ctypes.c_float), ("vr_epsilon", ctypes.c_float),
+        ("max_value", ctypes.c_float),
     ]
 
 
@@ -124,6 +134,18 @@ def load():
         getattr(lib, name).restype = ci
     lib.tf_watershed_flood_host.argtypes = [vp, vp, ll, vp, ci, vp, vp, vp, vp, vp, vp, ll]
     lib.tf_watershed_flood_host.restype = ci
+    dp = ctypes.POINTER(DisParams)
+    lib.tf_dis_default_params.argtypes = [dp, ci]
+    lib.tf_dis_default_params.restype = None
+    lib.tf_dis_scale_plan.argtypes = [ci, ci, dp, ctypes.POINTER(ci), ctypes.POINTER(ci), ctypes.POINTER(ci),
+                                      ctypes.POINTER(ci)]
+    lib.tf_dis_scale_plan.restype = ci
+    lib.tf_dis_workspace_bytes.argtypes = [ci, ci, ci, dp]
+    lib.tf_dis_workspace_bytes.restype = sz
+    lib.tf_dis_pairs.argtypes = [vp, vp, vp, ll, vp, ll, ci, ci, ci, dp, vp, sz, vp]
+    lib.tf_dis_pairs.restype = ci
+    lib.tf_dis_scale_images.argtypes = [vp, ci, ci, ci, dp, ci, vp, vp, vp, vp, sz, vp]
+    lib.tf_dis_scale_images.restype = ci
     lib.tf_profile_enable.argtypes = [ci]
     lib.tf_profile_read.argtypes = [ci, ctypes.POINTER(cd), ctypes.POINTER(cd), ctypes.POINTER(ll)]
     for name in ("tf_profile_enable", "tf_profile_reset", "tf_profile_read", "tf_fb_level_plan", "tf_fb_poly_constants", "tf_pair_normalise_u8", "tf_farneback_pairs",
@@ -169,6 +191,16 @@ def poly_constants(params=None):
     out = (ctypes.c_float * 22)()
     check(load().tf_fb_poly_constants(ctypes.byref(params), out), "tf_fb_poly_constants")
     return np.array(out, dtype=np.float32)
+
+
+def dis_scale_plan(H, W, params):
+    """(finest, coarsest, {scale: (h, w)}) of a DIS call on an H x W frame; raises where OpenCV refuses the frame."""
+    f, c = ctypes.c_int(), ctypes.c_int()
+    hs = (ctypes.c_int * 16)()
+    ws = (ctypes.c_int * 16)()
+    check(load().tf_dis_scale_plan(H, W, ctypes.byref(params), ctypes.byref(f), ctypes.byref(c), hs, ws),
+          "tf_dis_scale_plan")
+    return f.value, c.value, {s: (hs[s], ws[s]) for s in range(f.value, c.value + 1)}
 
 
 def workspace_bytes(n_pairs, H, W, params=None):

@@ -694,7 +694,15 @@ except Exception:  # pragma: no cover
 # ------------------------------------------------------------------------------------------------------------------
 # flow construction
 # ------------------------------------------------------------------------------------------------------------------
-def _check_model(model: str, vr_steps: int):
+def _is_dis(model) -> bool:
+    from .dis import DISOpticalFlow
+    return isinstance(model, DISOpticalFlow)
+
+
+def _check_model(model, vr_steps: int):
+    """``model``: the reference's model name, or a :class:`tobac_flow_b200.DISOpticalFlow` instance."""
+    if _is_dis(model):
+        return
     if model not in _REFERENCE_MODELS:
         raise ValueError(  # utils/flow_utils.py:72-75
             "'model' parameter must be one of: 'Farneback', 'DeepFlow', 'PCA', 'SimpleFlow', 'SparseToDense', "
@@ -703,7 +711,7 @@ def _check_model(model: str, vr_steps: int):
         raise NotImplementedError(f"optical-flow model '{model}' is not built in tobac_flow_b200 (only 'Farneback')")
 
 
-def _pair_batch(n_pairs: int, H: int, W: int, params, vr: bool = False) -> int:
+def _pair_batch(n_pairs: int, H: int, W: int, params, vr: bool = False, model=None) -> int:
     """Pairs per launch batch: as many as fit comfortably in free HBM, at most 512 Mpx (larger batches amortise the wave
     quantisation and the latency-bound launches of the small pyramid levels: 28.4 vs 30.5 ms per 96 CONUS frames for
     the coarse levels at 512 vs 256 Mpx), in equally sized batches (a small last batch would run at a fraction of the
@@ -711,10 +719,12 @@ def _pair_batch(n_pairs: int, H: int, W: int, params, vr: bool = False) -> int:
     # (the answer for a shape is remembered: `cudaMemGetInfo` is a driver call that can wait milliseconds behind a
     # monitoring query -- nvidia-smi -- and it sits in front of a call's first kernel launch; a shape whose workspace
     # allocation fails later drops its entry, see calculate_flow_device)
-    key = (torch.cuda.current_device(), n_pairs, H, W, bool(vr), params.num_levels, os.environ.get("TF_PAIR_BATCH_MPX"))
+    dis = _is_dis(model)
+    key = (torch.cuda.current_device(), n_pairs, H, W, bool(vr), model.key() if dis else params.num_levels,
+           os.environ.get("TF_PAIR_BATCH_MPX"))
     if key in _PAIR_BATCH_CACHE:
         return _PAIR_BATCH_CACHE[key]
-    per_pair = _lib.workspace_bytes(1, H, W, params) + 2 * H * W
+    per_pair = (model.workspace_bytes(1, H, W) if dis else _lib.workspace_bytes(1, H, W, params)) + 2 * H * W
     if vr:
         per_pair += int(_lib.load().tf_vr_workspace_bytes(1, H, W))
     free, _ = torch.cuda.mem_get_info()
@@ -733,12 +743,14 @@ _PAIR_BATCH_CACHE = {}
 def calculate_flow_device(frames: torch.Tensor, fwd: torch.Tensor, bwd: torch.Tensor, smoothing_passes: int = 0,
                           interp_method: str = "linear", max_value: float | None = None,
                           next_frames: torch.Tensor | None = None, batch: int | None = None, vr_steps: int = 0,
-                          frames_ready: Callable | None = None, batch_plan=None, batch_done: Callable | None = None) -> None:
+                          frames_ready: Callable | None = None, batch_plan=None, batch_done: Callable | None = None,
+                          model=None) -> None:
     """Fill ``fwd[i]`` and ``bwd[i + 1]`` for every consecutive pair of ``frames`` (device tensors, in place).
 
     ``frames`` (T, H, W) float32 or float64; ``fwd``/``bwd`` (>= T, H, W, 2) float32.  With ``next_frames`` the pairs are
     (frames[i], next_frames[i]) and results go to fwd[i], bwd[i + 1] for every i (``calculate_flow_2``).
     ``max_value`` fuses the clamp of ``create_flow`` into the last kernel when no smoothing follows.
+    ``model``: None (Farneback) or a :class:`tobac_flow_b200.DISOpticalFlow`.
     """
     lib = _lib.load()
     T, H, W = frames.shape
@@ -748,8 +760,11 @@ def calculate_flow_device(frames: torch.Tensor, fwd: torch.Tensor, bwd: torch.Te
     interp = _interp_code(interp_method)
     use_vr = bool(vr_steps) and vr_steps > 0   # flow.py:513-519: one refinement whenever vr_steps > 0
     fuse_clamp = (max_value is not None) and smoothing_passes == 0 and not use_vr
+    dis = _is_dis(model)
     params = _lib.default_params(max_value if fuse_clamp else 0.0)
-    nb = batch or _pair_batch(n_pairs, H, W, params, use_vr)
+    if dis:
+        dis_params = model.params(max_value if fuse_clamp else 0.0)
+    nb = batch or _pair_batch(n_pairs, H, W, params, use_vr, model)
     if batch_plan is None:
         batch_plan = [min(nb, n_pairs - p0) for p0 in range(0, n_pairs, nb)]
     nb = max(batch_plan)
@@ -761,7 +776,7 @@ def calculate_flow_device(frames: torch.Tensor, fwd: torch.Tensor, bwd: torch.Te
     f64 = frames.dtype == torch.float64        # float64 frames are normalised in float64, as numpy does for the reference
     mm = torch.empty((2 * nb,), dtype=frames.dtype, device=dev)
     normalise = lib.tf_pair_normalise_u8_f64 if f64 else lib.tf_pair_normalise_u8
-    ws_bytes = _lib.workspace_bytes(nb, H, W, params)
+    ws_bytes = model.workspace_bytes(nb, H, W) if dis else _lib.workspace_bytes(nb, H, W, params)
     try:
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
     except torch.cuda.OutOfMemoryError:
@@ -790,8 +805,12 @@ def calculate_flow_device(frames: torch.Tensor, fwd: torch.Tensor, bwd: torch.Te
                    "tf_pair_normalise_u8")
         fo = fwd.data_ptr() + p0 * hw * 2 * 4
         bo = bwd.data_ptr() + (p0 + 1) * hw * 2 * 4
-        _lib.check(lib.tf_farneback_pairs(q0.data_ptr(), q1.data_ptr(), fo, hw * 2, bo, hw * 2, n, H, W,
-                                          ctypes.byref(params), ws.data_ptr(), ws_bytes, st), "tf_farneback_pairs")
+        if dis:
+            _lib.check(lib.tf_dis_pairs(q0.data_ptr(), q1.data_ptr(), fo, hw * 2, bo, hw * 2, n, H, W,
+                                        ctypes.byref(dis_params), ws.data_ptr(), ws_bytes, st), "tf_dis_pairs")
+        else:
+            _lib.check(lib.tf_farneback_pairs(q0.data_ptr(), q1.data_ptr(), fo, hw * 2, bo, hw * 2, n, H, W,
+                                              ctypes.byref(params), ws.data_ptr(), ws_bytes, st), "tf_farneback_pairs")
         if use_vr:
             _lib.check(lib.tf_variational_refinement(q0.data_ptr(), q1.data_ptr(), fo, hw * 2, bo, hw * 2, n, H, W,
                                                      ctypes.byref(vr_params), vr_ws.data_ptr(), vr_bytes, st),
@@ -871,7 +890,7 @@ def _calculate_flow_tensors(data, model, vr_steps, smoothing_passes, interp_meth
         plan = batch_done = None
         if host_plan:
             use_vr = bool(vr_steps) and vr_steps > 0
-            plan = _host_batch_plan(T - 1, _pair_batch(T - 1, H, W, _lib.default_params(0.0), use_vr))
+            plan = _host_batch_plan(T - 1, _pair_batch(T - 1, H, W, _lib.default_params(0.0), use_vr, model))
             if max_value is not None and max_value != 0 and smoothing_passes == 0 and not use_vr:
                 # the clamp is fused into the last iteration kernel, so a batch's vectors are final once the end rules of
                 # the first / last frame (flow.py:425-426) are applied: do that with the batch that computes them and mark
@@ -892,11 +911,12 @@ def _calculate_flow_tensors(data, model, vr_steps, smoothing_passes, interp_meth
                     # vectors of frames [0, p0 + n) are final: fwd[i] comes from pair i, bwd[i] from pair i - 1
                     ready.append((T if last else p0 + n, ev))
         calculate_flow_device(frames, fwd, bwd, smoothing_passes, interp_method, max_value, vr_steps=vr_steps,
-                              batch=batch, frames_ready=frames_ready, batch_plan=plan, batch_done=batch_done)
+                              batch=batch, frames_ready=frames_ready, batch_plan=plan, batch_done=batch_done,
+                              model=model)
     else:
         # calculate_flow_2 (flow.py:431-496): pairs (a[i], b[i]) for i < T-1
         calculate_flow_device(frames[:T - 1], fwd, bwd, smoothing_passes, interp_method, max_value,
-                              next_frames=frames_b[:T - 1], vr_steps=vr_steps)
+                              next_frames=frames_b[:T - 1], vr_steps=vr_steps, model=model)
     clamp_all = max_value is not None and (smoothing_passes > 0 or (bool(vr_steps) and vr_steps > 0))
     if not early_final:
         finalise_flow_device(fwd, bwd, max_value, clamp_all)
@@ -931,6 +951,9 @@ def calculate_flow_2(a, b, model: str = "Farneback", vr_steps: int = 0, smoothin
 def create_flow(data, model: str = "Farneback", vr_steps: int = 0, smoothing_passes: int = 0,
                 interp_method: str = "linear", max_value=20) -> Flow:
     """``create_flow`` (tobac_flow/flow.py:23-65): flow vectors for ``data`` (t, y, x), clamped to +-max_value.
+
+    ``model`` is "Farneback" or a :class:`tobac_flow_b200.DISOpticalFlow` (as for ``calculate_flow`` /
+    ``calculate_flow_2``).
 
     The returned ``Flow`` keeps the vectors on the GPU.
     """
