@@ -9,6 +9,7 @@ import torch
 
 from . import _lib
 from .flow import _device, _stream, _to_host
+from .label import relabel_device
 
 
 def _labels_device(labels):
@@ -33,15 +34,18 @@ def _mask_device(mask, shape):
     return m.to(torch.uint8).contiguous()
 
 
-def label_stats_device(labels: torch.Tensor, mask_a=None, mask_b=None):
-    """(n_labels, tmin, tmax, any_a, any_b) as host arrays of n_labels + 1 entries for a (T, ...) int32 CUDA tensor."""
+def label_stats_device(labels: torch.Tensor, mask_a=None, mask_b=None, n_labels=None):
+    """(n_labels, tmin, tmax, any_a, any_b) as host arrays of n_labels + 1 entries for a (T, ...) int32 CUDA tensor
+    (tmax = -1 and tmin huge where a label does not occur).  ``n_labels`` defaults to the largest label, which costs a
+    device reduction and a host sync."""
     lib = _lib.load()
     dev = labels.device
     T = labels.shape[0]
     hw = labels.numel() // max(T, 1)
-    mx = torch.zeros((1,), dtype=torch.int32, device=dev)
-    _lib.check(lib.tf_label_max(labels.data_ptr(), labels.numel(), mx.data_ptr(), _stream()), "tf_label_max")
-    n_labels = int(mx.item())
+    if n_labels is None:
+        mx = torch.zeros((1,), dtype=torch.int32, device=dev)
+        _lib.check(lib.tf_label_max(labels.data_ptr(), labels.numel(), mx.data_ptr(), _stream()), "tf_label_max")
+        n_labels = int(mx.item())
     stats = torch.empty((4, n_labels + 1), dtype=torch.int32, device=dev)
     _lib.check(lib.tf_label_stats(labels.data_ptr(), mask_a.data_ptr() if mask_a is not None else None,
                                   mask_b.data_ptr() if mask_b is not None else None, T, hw, n_labels,
@@ -51,15 +55,15 @@ def label_stats_device(labels: torch.Tensor, mask_a=None, mask_b=None):
     return n_labels, s[0], s[1], s[2], s[3]
 
 
-def _apply_keep(labels: torch.Tensor, n_labels: int, wh: np.ndarray) -> torch.Tensor:
-    remap = np.zeros(n_labels + 1, np.int32)
+def _keep_table(wh: np.ndarray) -> np.ndarray:
+    """Relabel table over labels 0..len(wh): drops label i + 1 where ``wh[i]`` is False, numbers the rest 1, 2, ..."""
+    remap = np.zeros(len(wh) + 1, np.int32)
     remap[1:] = np.cumsum(wh) * wh                                  # analysis.py:72-73
-    out = torch.empty_like(labels)
-    if labels.numel():
-        map_d = torch.from_numpy(remap).to(labels.device)
-        _lib.check(_lib.load().tf_relabel(labels.data_ptr(), map_d.data_ptr(), out.data_ptr(), labels.numel(), n_labels,
-                                          _stream()), "tf_relabel")
-    return out
+    return remap
+
+
+def _apply_keep(labels: torch.Tensor, wh: np.ndarray) -> torch.Tensor:
+    return relabel_device(labels, _keep_table(wh))
 
 
 def _finish(out, host, np_dtype):
@@ -71,29 +75,29 @@ def _finish(out, host, np_dtype):
 def filter_labels_by_length(labels, min_length):
     """analysis.py:66-75: keep labels whose extent along axis 0 (ndi.find_objects) is >= min_length; renumber."""
     lab, host, np_dtype = _labels_device(labels)
-    n_labels, tmin, tmax, _, _ = label_stats_device(lab)
+    _, tmin, tmax, _, _ = label_stats_device(lab)
     if (tmax[1:] < 0).any():
         raise TypeError("'NoneType' object is not subscriptable")   # ndi.find_objects gives None for absent labels
     wh = (tmax[1:] - tmin[1:] + 1) >= min_length
-    return _finish(_apply_keep(lab, n_labels, wh), host, np_dtype)
+    return _finish(_apply_keep(lab, wh), host, np_dtype)
 
 
 def filter_labels_by_mask(labels, mask):
     """analysis.py:78-86: keep labels with at least one pixel inside ``mask``; renumber."""
     lab, host, np_dtype = _labels_device(labels)
     m = _mask_device(mask, lab.shape)
-    n_labels, _, _, any_a, _ = label_stats_device(lab, m)
+    _, _, _, any_a, _ = label_stats_device(lab, m)
     wh = any_a[1:] != 0
-    return _finish(_apply_keep(lab, n_labels, wh), host, np_dtype)
+    return _finish(_apply_keep(lab, wh), host, np_dtype)
 
 
 def filter_labels_by_length_and_mask(labels, mask, min_length):
     """analysis.py:89-102."""
     lab, host, np_dtype = _labels_device(labels)
     m = _mask_device(mask, lab.shape)
-    n_labels, tmin, tmax, any_a, _ = label_stats_device(lab, m)
+    _, tmin, tmax, any_a, _ = label_stats_device(lab, m)
     wh = np.logical_and((tmax[1:] - tmin[1:] + 1) >= min_length, any_a[1:] != 0)
-    return _finish(_apply_keep(lab, n_labels, wh), host, np_dtype)
+    return _finish(_apply_keep(lab, wh), host, np_dtype)
 
 
 def filter_labels_by_length_and_multimask_legacy(labels, masks, min_length):
@@ -103,16 +107,15 @@ def filter_labels_by_length_and_multimask_legacy(labels, masks, min_length):
         raise ValueError("masks input must be a list of masks to process")
     lab, host, np_dtype = _labels_device(labels)
     wh = None
-    n_labels = 0
     ms = [_mask_device(m, lab.shape) for m in masks]
     for k in range(0, max(len(ms), 1), 2):
         ma = ms[k] if k < len(ms) else None
         mb = ms[k + 1] if k + 1 < len(ms) else None
-        n_labels, tmin, tmax, any_a, any_b = label_stats_device(lab, ma, mb)
+        _, tmin, tmax, any_a, any_b = label_stats_device(lab, ma, mb)
         ok = (tmax[1:] - tmin[1:] + 1) >= min_length
         if ma is not None:
             ok = np.logical_and(ok, any_a[1:] != 0)
         if mb is not None:
             ok = np.logical_and(ok, any_b[1:] != 0)
         wh = ok if wh is None else np.logical_and(wh, ok)
-    return _finish(_apply_keep(lab, n_labels, wh), host, np_dtype)
+    return _finish(_apply_keep(lab, wh), host, np_dtype)

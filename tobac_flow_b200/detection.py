@@ -80,9 +80,8 @@ def curvature_filter_device(field: torch.Tensor, sigma=2, threshold=0, direction
         _lib.check(lib.tf_binary_fill_holes(m[done:].data_ptr(), filled[done:].data_ptr(), tc, H, W, ws.data_ptr(),
                                             ws_bytes, _stream()), "tf_binary_fill_holes")
         done += tc
-    _lib.check(lib.tf_binary_opening_cross(filled.data_ptr(), m.data_ptr(), T, H, W, _stream()),
-               "tf_binary_opening_cross")
-    return m
+    del m
+    return _binary_opening(filled)
 
 
 def get_curvature_filter(field, sigma=2, threshold=0, direction="negative"):
@@ -106,6 +105,62 @@ def grey_opening_cross_device(field: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def _threshold_ge(x: torch.Tensor, threshold) -> torch.Tensor:
+    """uint8 mask of ``x >= threshold`` for a contiguous float CUDA tensor."""
+    m = torch.empty(x.shape, dtype=torch.uint8, device=x.device)
+    _lib.check(_lib.load().tf_threshold_ge(x.data_ptr(), float(threshold), m.data_ptr(), _float_code(x), x.numel(),
+                                           _stream()), "tf_threshold_ge")
+    return m
+
+
+def _mask_multiply(x: torch.Tensor, mask: torch.Tensor) -> torch.Tensor:
+    """``x * mask`` for a float CUDA tensor and a uint8 mask of the same shape."""
+    out = torch.empty_like(x)
+    _lib.check(_lib.load().tf_mask_multiply(x.data_ptr(), mask.data_ptr(), out.data_ptr(), _float_code(x), x.numel(),
+                                            _stream()), "tf_mask_multiply")
+    return out
+
+
+def _binary_opening(m: torch.Tensor) -> torch.Tensor:
+    """Per-frame binary opening of a (T, H, W) uint8 mask with the 2-D cross."""
+    T, H, W = m.shape
+    out = torch.empty_like(m)
+    _lib.check(_lib.load().tf_binary_opening_cross(m.data_ptr(), out.data_ptr(), T, H, W, _stream()),
+               "tf_binary_opening_cross")
+    return out
+
+
+def scale_by_dt_device(raw32: torch.Tensor, dt_minutes) -> torch.Tensor:
+    """A (T, H, W) float32 ``Flow.diff`` result divided frame by frame by ``dt_minutes`` (T doubles) -> float64."""
+    T, H, W = raw32.shape
+    dt = torch.from_numpy(np.ascontiguousarray(np.asarray(dt_minutes, np.float64))).to(raw32.device)
+    assert dt.numel() == T
+    raw = torch.empty((T, H, W), dtype=torch.float64, device=raw32.device)
+    _lib.check(_lib.load().tf_scale_frames(raw32.data_ptr(), dt.data_ptr(), raw.data_ptr(), T, H, W, _stream()),
+               "tf_scale_frames")
+    return raw
+
+
+def growth_seed_masks_device(smoothed: torch.Tensor, wvd: torch.Tensor):
+    """detection.py:105-112 -> (filtered, filtered >= 0.5, wvd >= -5, seeds): ``filtered`` is the grey opening of
+    ``smoothed`` times the curvature filter of ``wvd``, the seeds are ``filtered >= 0.25`` opened; masks are uint8."""
+    opened = grey_opening_cross_device(smoothed)                                        # :105-107
+    curv = curvature_filter_device(wvd)                                                 # :108
+    filtered = _mask_multiply(opened, curv)
+    del opened, curv
+    seeds = _binary_opening(_threshold_ge(filtered, 0.25))
+    return filtered, _threshold_ge(filtered, 0.5), _threshold_ge(wvd, -5.0), seeds
+
+
+def growth_marker_keep(tmin, tmax, any_a, any_b) -> np.ndarray:
+    """detection.py:114-119 from the per-label statistics of the linked labels (``any_a``: touches filtered >= 0.5,
+    ``any_b``: touches wvd >= -5): the relabel table that keeps the labels lasting at least 3 frames and touching both
+    masks, numbered 1, 2, ... in label order.  The reference renumbers three times; dropping labels commutes with the
+    order-preserving renumbering, so one table does."""
+    wh = ((tmax[1:] - tmin[1:] + 1) >= 3) & (any_a[1:] != 0) & (any_b[1:] != 0)
+    return analysis._keep_table(wh)
+
+
 def time_diff_minutes(t_coord) -> np.ndarray:
     """``get_time_diff_from_coord`` (tobac_flow/utils/datetime_utils.py:126-166): centred differences in minutes."""
     import pandas as pd
@@ -118,41 +173,13 @@ def time_diff_minutes(t_coord) -> np.ndarray:
 def growth_markers_device(flow: Flow, wvd: torch.Tensor, dt_minutes) -> dict:
     """The whole of detection.py:98-118 on device tensors; returns the intermediates the reference exposes plus the
     markers.  ``wvd`` (T, H, W) float32 or float64 CUDA tensor, ``dt_minutes`` T doubles."""
-    lib = _lib.load()
-    dev = wvd.device
-    T, H, W = wvd.shape
-    n = wvd.numel()
-    st = _stream
-    raw32 = flow.diff(wvd)                                                              # detection.py:99
-    dt = torch.from_numpy(np.ascontiguousarray(np.asarray(dt_minutes, np.float64))).to(dev)
-    assert dt.numel() == T
-    raw = torch.empty((T, H, W), dtype=torch.float64, device=dev)
-    _lib.check(lib.tf_scale_frames(raw32.data_ptr(), dt.data_ptr(), raw.data_ptr(), T, H, W, st()), "tf_scale_frames")
-    del raw32
+    raw = scale_by_dt_device(flow.diff(wvd), dt_minutes)                                # detection.py:99-100
     smoothed = filtered_tdiff(flow, raw)                                                # :103, float32
-    opened = grey_opening_cross_device(smoothed)                                        # :105-107
-    curv = curvature_filter_device(wvd)                                                 # :108
-    filtered = torch.empty_like(opened)
-    _lib.check(lib.tf_mask_multiply(opened.data_ptr(), curv.data_ptr(), filtered.data_ptr(), _float_code(opened), n,
-                                    st()), "tf_mask_multiply")
-    del opened, curv
-    m025 = torch.empty((T, H, W), dtype=torch.uint8, device=dev)
-    m05 = torch.empty_like(m025)
-    warm = torch.empty_like(m025)
-    _lib.check(lib.tf_threshold_ge(filtered.data_ptr(), 0.25, m025.data_ptr(), _float_code(filtered), n, st()),
-               "tf_threshold_ge")
-    _lib.check(lib.tf_threshold_ge(filtered.data_ptr(), 0.5, m05.data_ptr(), _float_code(filtered), n, st()),
-               "tf_threshold_ge")
-    _lib.check(lib.tf_threshold_ge(wvd.data_ptr(), -5.0, warm.data_ptr(), _float_code(wvd), n, st()), "tf_threshold_ge")
-    seeds = torch.empty_like(m025)
-    _lib.check(lib.tf_binary_opening_cross(m025.data_ptr(), seeds.data_ptr(), T, H, W, st()), "tf_binary_opening_cross")
+    filtered, m05, warm, seeds = growth_seed_masks_device(smoothed, wvd)                # :105-112
     flat, n_flat = _label.flat_label_device(seeds, 1)                                   # Flow.label -> label.py:125
     linked, _ = _label.link_overlap_device(flow, flat, _label._default_structure(), 0, 1, n_flat)
-    # :114-119: length >= 3, then touches (filtered >= 0.5), then touches (wvd >= -5); three renumberings in the
-    # reference, composed here into one (dropping labels commutes with the order-preserving renumbering)
-    n_labels, tmin, tmax, any_a, any_b = analysis.label_stats_device(linked, m05, warm)
-    wh = ((tmax[1:] - tmin[1:] + 1) >= 3) & (any_a[1:] != 0) & (any_b[1:] != 0)
-    markers = analysis._apply_keep(linked, n_labels, wh)
+    _, tmin, tmax, any_a, any_b = analysis.label_stats_device(linked, m05, warm)
+    markers = _label.relabel_device(linked, growth_marker_keep(tmin, tmax, any_a, any_b))   # :114-119
     return dict(raw=raw, smoothed=smoothed, filtered=filtered, seeds=seeds, flat=flat, linked=linked, markers=markers)
 
 
@@ -166,14 +193,7 @@ def _time_coord(field):
 def growth_rate_device(flow: Flow, field: torch.Tensor, dt_minutes, method: str = "linear") -> torch.Tensor:
     """``get_growth_rate`` on a float32 / float64 CUDA tensor: Flow.diff / dt, then the 5-point same-step nanmean
     (float32 result)."""
-    T, H, W = field.shape
-    raw32 = flow.diff(field, method=method)
-    dt = torch.from_numpy(np.ascontiguousarray(np.asarray(dt_minutes, np.float64))).to(field.device)
-    assert dt.numel() == T
-    raw = torch.empty((T, H, W), dtype=torch.float64, device=field.device)
-    _lib.check(_lib.load().tf_scale_frames(raw32.data_ptr(), dt.data_ptr(), raw.data_ptr(), T, H, W, _stream()),
-               "tf_scale_frames")
-    del raw32
+    raw = scale_by_dt_device(flow.diff(field, method=method), dt_minutes)
     s_struct = np.zeros((3, 3, 3), bool)
     s_struct[1, 1, :] = s_struct[1, :, 1] = True
     return flow.convolve(raw, structure=s_struct, func=_nanmean0, method=method)
@@ -193,19 +213,11 @@ def get_growth_rate(flow, field, method: str = "linear"):
 def anvil_markers_device(flow: Flow, field: torch.Tensor, threshold=-5, overlap=0.5, absolute_overlap=5,
                          min_length=3) -> torch.Tensor:
     """``get_anvil_markers`` on a float CUDA tensor (subsegment_shrink == 0)."""
-    lib = _lib.load()
-    T, H, W = field.shape
-    m = torch.empty((T, H, W), dtype=torch.uint8, device=field.device)
-    _lib.check(lib.tf_threshold_ge(field.data_ptr(), float(threshold), m.data_ptr(), _float_code(field), field.numel(),
-                                   _stream()), "tf_threshold_ge")
-    opened = torch.empty_like(m)
-    _lib.check(lib.tf_binary_opening_cross(m.data_ptr(), opened.data_ptr(), T, H, W, _stream()), "tf_binary_opening_cross")
-    del m
-    flat, n_flat = _label.flat_label_device(opened, 1)
+    flat, n_flat = _label.flat_label_device(_binary_opening(_threshold_ge(field, threshold)), 1)
     linked, _ = _label.link_overlap_device(flow, flat, _label._default_structure(), overlap, absolute_overlap, n_flat)
-    n_labels, tmin, tmax, _, _ = analysis.label_stats_device(linked)
+    _, tmin, tmax, _, _ = analysis.label_stats_device(linked)
     wh = (tmax[1:] - tmin[1:] + 1) > min_length        # find_object_lengths(...) > min_length, then remap_labels
-    return analysis._apply_keep(linked, n_labels, wh)
+    return analysis._apply_keep(linked, wh)
 
 
 def get_anvil_markers(flow, field, threshold=-5, overlap=0.5, absolute_overlap=5, subsegment_shrink=0, min_length=3):
@@ -287,43 +299,18 @@ def growth_markers_multichannel_device(flow: Flow, wvd: torch.Tensor, bt: torch.
                                        min_length=4, lower_threshold=0.25, upper_threshold=0.5) -> dict:
     """detection.py:203-254 on device tensors (``subsegment_shrink == 0``): growth of the water-vapour difference OR
     cooling of the window brightness temperature, each inside its curvature filter."""
-    lib = _lib.load()
-    dev = wvd.device
-    T, H, W = wvd.shape
-    n = wvd.numel()
-    st = _stream
-
-    def smoothed_rate(field, dt_minutes):
-        raw32 = flow.diff(field)
-        dt = torch.from_numpy(np.ascontiguousarray(np.asarray(dt_minutes, np.float64))).to(dev)
-        assert dt.numel() == T
-        raw = torch.empty((T, H, W), dtype=torch.float64, device=dev)
-        _lib.check(lib.tf_scale_frames(raw32.data_ptr(), dt.data_ptr(), raw.data_ptr(), T, H, W, st()), "tf_scale_frames")
-        return filtered_tdiff(flow, raw)
-
-    def times_mask(x, mask):
-        out = torch.empty_like(x)
-        _lib.check(lib.tf_mask_multiply(x.data_ptr(), mask.data_ptr(), out.data_ptr(), _float_code(x), n, st()),
-                   "tf_mask_multiply")
-        return out
-
-    def ge(x, thr):
-        m = torch.empty((T, H, W), dtype=torch.uint8, device=dev)
-        _lib.check(lib.tf_threshold_ge(x.data_ptr(), float(thr), m.data_ptr(), _float_code(x), n, st()), "tf_threshold_ge")
-        return m
-
-    wvd_s = smoothed_rate(wvd, dt_wvd)                                                  # :214-217
-    bt_s = smoothed_rate(bt, dt_bt)                                                     # :218-220
-    grow = ge(times_mask(wvd_s, curvature_filter_device(wvd)), lower_threshold)         # :223
-    cool = ge(-times_mask(bt_s, curvature_filter_device(bt, direction="positive")), lower_threshold)   # :224-225 (x <= -l)
-    seeds_in = torch.bitwise_or(grow, cool)
-    seeds = torch.empty_like(seeds_in)
-    _lib.check(lib.tf_binary_opening_cross(seeds_in.data_ptr(), seeds.data_ptr(), T, H, W, st()), "tf_binary_opening_cross")
+    wvd_s = filtered_tdiff(flow, scale_by_dt_device(flow.diff(wvd), dt_wvd))           # :214-217
+    bt_s = filtered_tdiff(flow, scale_by_dt_device(flow.diff(bt), dt_bt))              # :218-220
+    grow = _threshold_ge(_mask_multiply(wvd_s, curvature_filter_device(wvd)), lower_threshold)     # :223
+    cool = _threshold_ge(-_mask_multiply(bt_s, curvature_filter_device(bt, direction="positive")),
+                         lower_threshold)                                               # :224-225 (x <= -l)
+    seeds = _binary_opening(torch.bitwise_or(grow, cool))
     flat, n_flat = _label.flat_label_device(seeds, 1)                                   # Flow.label(overlap=overlap), :227-233
     linked, _ = _label.link_overlap_device(flow, flat, _label._default_structure(), overlap, 1, n_flat)
     markers = linked
     if bool((linked != 0).any()):                                                       # :236-246
-        masks = [ge(wvd_s, upper_threshold), ge(-bt_s, upper_threshold), (wvd > -5).to(torch.uint8)]
+        masks = [_threshold_ge(wvd_s, upper_threshold), _threshold_ge(-bt_s, upper_threshold),
+                 (wvd > -5).to(torch.uint8)]
         markers = analysis.filter_labels_by_length_and_multimask_legacy(linked, masks, min_length)
     else:
         import warnings

@@ -50,13 +50,8 @@ class CudaOps:
 
     def overlap_table(self, flat_view, fwd, bwd, label_struct, has_prev, has_next, n_labels):
         """(keys, counts, sizes) of this rank's frames; ``flat_view`` carries the halo frames that exist."""
-        from . import _lib
-        from .flow import convolve_device
-        from .label import overlap_table_device
-        taps = convolve_device(flat_view, fwd, bwd, label_struct, "nearest", 0, np.int32, _lib.TF_RED_NONE,
-                               has_prev, has_next)
-        local = flat_view[int(has_prev):flat_view.shape[0] - int(has_next)].contiguous()
-        return overlap_table_device(local, taps[0], taps[1], n_labels)
+        from .label import warped_overlap_table_device
+        return warped_overlap_table_device(flat_view, fwd, bwd, label_struct, n_labels, has_prev, has_next)
 
     def relabel(self, flat, mapping):
         from .label import relabel_device
@@ -64,49 +59,19 @@ class CudaOps:
 
     # -- growth-marker detection (the per-frame filters of detection.py:98-118 are local to a rank) -------------------
     def scale_frames(self, raw32, dt_minutes):
-        from . import _lib
-        from .flow import _stream
-        T, H, W = raw32.shape
-        dt = torch.from_numpy(np.ascontiguousarray(np.asarray(dt_minutes, np.float64))).to(raw32.device)
-        out = torch.empty((T, H, W), dtype=torch.float64, device=raw32.device)
-        _lib.check(_lib.load().tf_scale_frames(raw32.data_ptr(), dt.data_ptr(), out.data_ptr(), T, H, W, _stream()),
-                   "tf_scale_frames")
-        return out
+        from .detection import scale_by_dt_device
+        return scale_by_dt_device(raw32, dt_minutes)
 
     def growth_seed_masks(self, smoothed, wvd):
         """(filtered >= 0.5, wvd >= -5, opened(filtered >= 0.25)) as uint8 tensors: detection.py:105-119."""
-        from . import _lib
-        from .detection import curvature_filter_device, grey_opening_cross_device, _float_code
-        from .flow import _stream
-        lib = _lib.load()
-        T, H, W = smoothed.shape
-        n = smoothed.numel()
-        opened = grey_opening_cross_device(smoothed)
-        curv = curvature_filter_device(wvd)
-        filtered = torch.empty_like(opened)
-        _lib.check(lib.tf_mask_multiply(opened.data_ptr(), curv.data_ptr(), filtered.data_ptr(), _float_code(opened), n,
-                                        _stream()), "tf_mask_multiply")
-        m025, m05, warm, seeds = (torch.empty((T, H, W), dtype=torch.uint8, device=smoothed.device) for _ in range(4))
-        for src, thr, dst in ((filtered, 0.25, m025), (filtered, 0.5, m05), (wvd, -5.0, warm)):
-            _lib.check(lib.tf_threshold_ge(src.data_ptr(), thr, dst.data_ptr(), _float_code(src), n, _stream()),
-                       "tf_threshold_ge")
-        _lib.check(lib.tf_binary_opening_cross(m025.data_ptr(), seeds.data_ptr(), T, H, W, _stream()),
-                   "tf_binary_opening_cross")
-        return m05, warm, seeds
+        from .detection import growth_seed_masks_device
+        return growth_seed_masks_device(smoothed, wvd)[1:]
 
     def label_stats(self, labels, mask_a, mask_b, n_labels):
         """(tmin, tmax, any_a, any_b) host arrays of n_labels + 1 entries over this rank's frames (local frame indices;
         tmax = -1 and tmin huge where the label does not occur here)."""
-        from . import _lib
-        from .flow import _stream
-        T = labels.shape[0]
-        hw = labels.numel() // max(T, 1)
-        st = torch.empty((4, n_labels + 1), dtype=torch.int32, device=labels.device)
-        _lib.check(_lib.load().tf_label_stats(labels.data_ptr(), mask_a.data_ptr(), mask_b.data_ptr(), T, hw, n_labels,
-                                              st[0].data_ptr(), st[1].data_ptr(), st[2].data_ptr(), st[3].data_ptr(),
-                                              _stream()), "tf_label_stats")
-        h = st.cpu().numpy()
-        return h[0], h[1], h[2], h[3]
+        from .analysis import label_stats_device
+        return label_stats_device(labels, mask_a, mask_b, n_labels)[1:]
 
 
 _HALO_STREAMS = {}
@@ -248,12 +213,12 @@ class ShardedFlow:
         frames (get_time_diff_from_coord evaluated on the whole series, sliced), ``t0`` its first global frame index.
         Exchanges: one-frame halos of the field and of the raw derivative (point to point), the labelling exchange of
         ``label``, and a min / max reduction of the per-label time extent and mask hits (one int per label)."""
+        from . import _lib
+        from .detection import _T_STRUCT, growth_marker_keep
         ops = self.ops
-        s_t = np.zeros((3, 3, 3))
-        s_t[:, 1, 1] = 1
-        raw32 = self.convolve(wvd, s_t, reducer=1)                                     # Flow.diff       (:99)
+        raw32 = self.convolve(wvd, _T_STRUCT, reducer=_lib.TF_RED_DIFF)                # Flow.diff       (:99)
         raw = make_shard(ops.scale_frames(raw32, dt_minutes_local), self.rank, self.world)   # / dt      (:100)
-        smoothed = self.convolve(raw, s_t, reducer=2)                                  # filtered_tdiff  (:103)
+        smoothed = self.convolve(raw, _T_STRUCT, reducer=_lib.TF_RED_NANMEAN)          # filtered_tdiff  (:103)
         m05, warm, seeds = ops.growth_seed_masks(smoothed, wvd.local.contiguous())     # :105-112
         linked, n_obj = self.label(seeds, overlap=0.0, absolute_overlap=1, return_count=True)
         tmin, tmax, any_a, any_b = ops.label_stats(linked, m05, warm, n_obj)
@@ -266,10 +231,7 @@ class ShardedFlow:
             dist.all_reduce(lo, op=dist.ReduceOp.MIN, group=self.group)
             dist.all_reduce(hi, op=dist.ReduceOp.MAX, group=self.group)
         lo, hi = lo.cpu().numpy(), hi.cpu().numpy()
-        wh = ((hi[0, 1:] - lo[1:] + 1) >= 3) & (hi[1, 1:] != 0) & (hi[2, 1:] != 0)     # :114-119
-        remap = np.zeros(n_obj + 1, np.int32)
-        remap[1:] = np.cumsum(wh) * wh
-        return smoothed, ops.relabel(linked, remap)
+        return smoothed, ops.relabel(linked, growth_marker_keep(lo, hi[0], hi[1], hi[2]))   # :114-119
 
 
 def create_flow_sharded(shard: Shard, smoothing_passes=0, interp_method="linear", max_value=20, ops=None, group=None,

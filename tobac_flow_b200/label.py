@@ -119,6 +119,17 @@ def overlap_table_device(flat: torch.Tensor, back: torch.Tensor, fwd: torch.Tens
     return k_h, c_h, sizes.cpu().numpy()
 
 
+def warped_overlap_table_device(flat_view: torch.Tensor, fwd: torch.Tensor, bwd: torch.Tensor, label_struct,
+                                n_labels: int, has_prev: bool = False, has_next: bool = False):
+    """``overlap_table_device`` of the flat labels against their neighbouring frames warped along the flow (nearest,
+    label.py:131-134).  With ``has_prev`` / ``has_next`` the first / last frame of ``flat_view`` is a halo frame of a
+    time shard: it is only warped, and the table covers the frames between the halos."""
+    taps = convolve_device(flat_view, fwd, bwd, label_struct, "nearest", 0, np.int32, _lib.TF_RED_NONE, has_prev,
+                           has_next)
+    local = flat_view[int(has_prev):flat_view.shape[0] - int(has_next)].contiguous()
+    return overlap_table_device(local, taps[0], taps[1], n_labels)
+
+
 def link_groups_host(keys: np.ndarray, counts: np.ndarray, sizes: np.ndarray, n_labels: int, overlap: float,
                      absolute_overlap: int):
     """tf_label_link_groups (the order-dependent walk of label.py:139-163, run on the host inside the library) ->
@@ -136,7 +147,7 @@ def link_groups_host(keys: np.ndarray, counts: np.ndarray, sizes: np.ndarray, n_
 
 def relabel_device(flat: torch.Tensor, mapping: np.ndarray) -> torch.Tensor:
     """out = mapping[flat] on the device (label.py:165-170)."""
-    out = torch.zeros_like(flat)
+    out = torch.empty_like(flat)                                 # tf_relabel writes every element
     if flat.numel():
         map_d = torch.from_numpy(np.ascontiguousarray(mapping, dtype=np.int32)).to(flat.device)
         _lib.check(_lib.load().tf_relabel(flat.data_ptr(), map_d.data_ptr(), out.data_ptr(), flat.numel(),
@@ -158,9 +169,8 @@ def link_overlap_device(flow, flat: torch.Tensor, structure, overlap: float, abs
         n_labels = int(mx.item())
         if bool((flat < 0).any()):
             raise ValueError("flat labels must be non-negative")                      # np.bincount raises the same
-    taps = convolve_device(flat, flow.forward_flow_device, flow.backward_flow_device, _label_struct(structure),
-                           "nearest", 0, np.int32, _lib.TF_RED_NONE)
-    keys, counts, sizes = overlap_table_device(flat, taps[0], taps[1], n_labels)
+    keys, counts, sizes = warped_overlap_table_device(flat, flow.forward_flow_device, flow.backward_flow_device,
+                                                      _label_struct(structure), n_labels)
     mapping, n_obj = link_groups_host(keys, counts, sizes, n_labels, overlap, absolute_overlap)
     return relabel_device(flat, mapping), n_obj
 
