@@ -70,7 +70,7 @@ def test_flat_label_conus_size():
 @pytest.mark.parametrize("shape", [(3, 40, 50), (2, 33, 129), (1, 3, 3), (2, 1, 9)])
 def test_fill_holes_and_opening(shape):
     from tobac_flow_b200 import _lib
-    from tobac_flow_b200.flow import _stream
+    from tobac_flow_b200._io import stream as _stream
     lib = _lib.load()
     rng = np.random.default_rng(5)
     T, H, W = shape

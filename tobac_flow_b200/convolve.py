@@ -5,7 +5,8 @@ import numpy as np
 import torch
 
 from . import _lib
-from .flow import Flow, _default_structure, _interp_code, _to_device, convolve_device
+from ._io import to_device
+from .flow import Flow, _default_structure, _interp_code, convolve_device
 
 
 def convolve(data, forward_flow, backward_flow, structure=None, method: str = "linear", dtype: type = np.float32,
@@ -28,8 +29,8 @@ def warp_flow(img, flow, method: str = "linear", fill_value: float = np.nan, off
     offsets = np.atleast_2d(np.asarray(offsets)).astype(int)
     if np.abs(offsets).max(initial=0) > 1:
         raise NotImplementedError("warp_flow offsets outside {-1, 0, 1} are not built in tobac_flow_b200")
-    t, host = _to_device(img)
-    f, _ = _to_device(flow, torch.float32)
+    t, host = to_device(img)
+    f, _ = to_device(flow, torch.float32)
     H, W = t.shape
     structure = np.zeros((3, 3, 3), bool)
     for dx, dy in offsets:

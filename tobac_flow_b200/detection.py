@@ -11,7 +11,8 @@ import torch
 from . import _lib
 from . import analysis
 from . import label as _label
-from .flow import Flow, _as_numpy, _device, _stream, _to_device, _to_host
+from ._io import float_to_device, like_input, stream, to_caller, to_device, to_host
+from .flow import Flow
 
 _T_STRUCT = np.zeros([3, 3, 3])
 _T_STRUCT[:, 1, 1] = 1
@@ -56,7 +57,7 @@ def gaussian_filter_yx_device(field: torch.Tensor, sigma: float) -> torch.Tensor
     tmp, out = torch.empty_like(field), torch.empty_like(field)
     _lib.check(_lib.load().tf_gaussian_filter_yx(field.data_ptr(), tmp.data_ptr(), out.data_ptr(), _float_code(field),
                                                  T, H, W, w.ctypes.data_as(_lib.ctypes.POINTER(_lib.ctypes.c_double)),
-                                                 radius, _stream()), "tf_gaussian_filter_yx")
+                                                 radius, stream()), "tf_gaussian_filter_yx")
     return out
 
 
@@ -69,7 +70,7 @@ def curvature_filter_device(field: torch.Tensor, sigma=2, threshold=0, direction
     smoothed = gaussian_filter_yx_device(field, sigma)
     m = torch.empty((T, H, W), dtype=torch.uint8, device=field.device)
     _lib.check(lib.tf_curvature_mask(smoothed.data_ptr(), m.data_ptr(), _float_code(smoothed), T, H, W, float(threshold),
-                                     int(direction == "positive"), _stream()), "tf_curvature_mask")
+                                     int(direction == "positive"), stream()), "tf_curvature_mask")
     del smoothed
     filled = torch.empty_like(m)
     done = 0
@@ -78,7 +79,7 @@ def curvature_filter_device(field: torch.Tensor, sigma=2, threshold=0, direction
         ws_bytes = int(lib.tf_ccl_workspace_bytes(tc, H, W))
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=field.device)
         _lib.check(lib.tf_binary_fill_holes(m[done:].data_ptr(), filled[done:].data_ptr(), tc, H, W, ws.data_ptr(),
-                                            ws_bytes, _stream()), "tf_binary_fill_holes")
+                                            ws_bytes, stream()), "tf_binary_fill_holes")
         done += tc
     del m
     return _binary_opening(filled)
@@ -88,20 +89,18 @@ def get_curvature_filter(field, sigma=2, threshold=0, direction="negative"):
     """detection.py:64-94: Gaussian-smoothed second differences both beyond the threshold, holes filled, opened."""
     if direction not in ("negative", "positive"):
         raise ValueError("Direction must be either positive or negative")
-    t, host = _to_device(field)
+    t, host = to_device(field)
     if not t.dtype.is_floating_point:
         raise NotImplementedError("get_curvature_filter: integer fields are not supported")
-    if t.dtype not in (torch.float32, torch.float64):
-        t = t.to(torch.float32)
-    m = curvature_filter_device(t, sigma, threshold, direction)
-    return _to_host(m).view(np.bool_) if host else m.to(torch.bool)
+    m = curvature_filter_device(float_to_device(t, torch.float32)[0], sigma, threshold, direction)
+    return to_host(m).view(np.bool_) if host else m.to(torch.bool)
 
 
 def grey_opening_cross_device(field: torch.Tensor) -> torch.Tensor:
     T, H, W = field.shape
     tmp, out = torch.empty_like(field), torch.empty_like(field)
     _lib.check(_lib.load().tf_grey_opening_cross(field.data_ptr(), tmp.data_ptr(), out.data_ptr(), _float_code(field),
-                                                 T, H, W, _stream()), "tf_grey_opening_cross")
+                                                 T, H, W, stream()), "tf_grey_opening_cross")
     return out
 
 
@@ -109,7 +108,7 @@ def _threshold_ge(x: torch.Tensor, threshold) -> torch.Tensor:
     """uint8 mask of ``x >= threshold`` for a contiguous float CUDA tensor."""
     m = torch.empty(x.shape, dtype=torch.uint8, device=x.device)
     _lib.check(_lib.load().tf_threshold_ge(x.data_ptr(), float(threshold), m.data_ptr(), _float_code(x), x.numel(),
-                                           _stream()), "tf_threshold_ge")
+                                           stream()), "tf_threshold_ge")
     return m
 
 
@@ -117,7 +116,7 @@ def _mask_multiply(x: torch.Tensor, mask: torch.Tensor) -> torch.Tensor:
     """``x * mask`` for a float CUDA tensor and a uint8 mask of the same shape."""
     out = torch.empty_like(x)
     _lib.check(_lib.load().tf_mask_multiply(x.data_ptr(), mask.data_ptr(), out.data_ptr(), _float_code(x), x.numel(),
-                                            _stream()), "tf_mask_multiply")
+                                            stream()), "tf_mask_multiply")
     return out
 
 
@@ -125,7 +124,7 @@ def _binary_opening(m: torch.Tensor) -> torch.Tensor:
     """Per-frame binary opening of a (T, H, W) uint8 mask with the 2-D cross."""
     T, H, W = m.shape
     out = torch.empty_like(m)
-    _lib.check(_lib.load().tf_binary_opening_cross(m.data_ptr(), out.data_ptr(), T, H, W, _stream()),
+    _lib.check(_lib.load().tf_binary_opening_cross(m.data_ptr(), out.data_ptr(), T, H, W, stream()),
                "tf_binary_opening_cross")
     return out
 
@@ -136,7 +135,7 @@ def scale_by_dt_device(raw32: torch.Tensor, dt_minutes) -> torch.Tensor:
     dt = torch.from_numpy(np.ascontiguousarray(np.asarray(dt_minutes, np.float64))).to(raw32.device)
     assert dt.numel() == T
     raw = torch.empty((T, H, W), dtype=torch.float64, device=raw32.device)
-    _lib.check(_lib.load().tf_scale_frames(raw32.data_ptr(), dt.data_ptr(), raw.data_ptr(), T, H, W, _stream()),
+    _lib.check(_lib.load().tf_scale_frames(raw32.data_ptr(), dt.data_ptr(), raw.data_ptr(), T, H, W, stream()),
                "tf_scale_frames")
     return raw
 
@@ -202,12 +201,8 @@ def growth_rate_device(flow: Flow, field: torch.Tensor, dt_minutes, method: str 
 def get_growth_rate(flow, field, method: str = "linear"):
     """detection.py:168-198: growth / cooling rate of ``field`` (an array with a ``.t`` time coordinate)."""
     dt = _time_coord(field)
-    on_device = isinstance(field, torch.Tensor) and field.is_cuda
-    f, _ = _to_device(field if isinstance(field, torch.Tensor) else _as_numpy(field))
-    if f.dtype not in (torch.float32, torch.float64):     # the taps are warped in the field's own dtype (cv2.remap)
-        f = f.to(torch.float32)
-    r = growth_rate_device(flow, f, dt, method)
-    return r if on_device else _to_host(r)
+    f, host = float_to_device(field, torch.float32)     # the taps are warped in the field's own dtype (cv2.remap)
+    return to_caller(growth_rate_device(flow, f, dt, method), host)
 
 
 def anvil_markers_device(flow: Flow, field: torch.Tensor, threshold=-5, overlap=0.5, absolute_overlap=5,
@@ -225,12 +220,8 @@ def get_anvil_markers(flow, field, threshold=-5, overlap=0.5, absolute_overlap=5
     flow, labels no longer than ``min_length`` steps dropped and the rest renumbered."""
     if subsegment_shrink != 0:
         raise NotImplementedError("subsegment_shrink != 0 (skimage watershed sub-segmentation) is not built here")
-    on_device = isinstance(field, torch.Tensor) and field.is_cuda
-    f, _ = _to_device(field if isinstance(field, torch.Tensor) else _as_numpy(field))
-    if f.dtype not in (torch.float32, torch.float64):
-        f = f.to(torch.float32)
-    r = anvil_markers_device(flow, f, threshold, overlap, absolute_overlap, min_length)
-    return r if on_device else _to_host(r)
+    f, host = float_to_device(field, torch.float32)
+    return to_caller(anvil_markers_device(flow, f, threshold, overlap, absolute_overlap, min_length), host)
 
 
 def detect_growth_markers(flow, wvd):
@@ -244,20 +235,11 @@ def detect_growth_markers(flow, wvd):
     if t_coord is None:
         raise AttributeError("wvd needs a time coordinate `.t` (detection.py:100)")
     dt = time_diff_minutes(t_coord)
-    on_device = isinstance(wvd, torch.Tensor) and wvd.is_cuda
-    w, _ = _to_device(wvd if isinstance(wvd, torch.Tensor) else _as_numpy(wvd))
-    if w.dtype not in (torch.float32, torch.float64):     # a float64 field is filtered in float64, as scipy would
-        w = w.to(torch.float32)
+    w, host = float_to_device(wvd, torch.float32)       # a float64 field is filtered in float64, as scipy would
     r = growth_markers_device(flow, w, dt)
-    if on_device:
+    if not host:
         return r["smoothed"], r["markers"]
-    smoothed, markers = _to_host(r["smoothed"]), _to_host(r["markers"])
-    if hasattr(wvd, "coords") and hasattr(wvd, "dims") and not isinstance(wvd, np.ndarray):
-        try:
-            markers = type(wvd)(markers, wvd.coords, wvd.dims)                          # detection.py:121-123
-        except Exception:
-            pass
-    return smoothed, markers
+    return to_host(r["smoothed"]), like_input(wvd, to_host(r["markers"]))              # detection.py:121-123
 
 
 def nan_gaussian_filter(a, *args, propagate_nan=True, **kwargs):
@@ -267,9 +249,7 @@ def nan_gaussian_filter(a, *args, propagate_nan=True, **kwargs):
     if kwargs or len(args) != 1:
         raise NotImplementedError("nan_gaussian_filter: only the sigma argument of gaussian_filter is supported")
     sigma = args[0]
-    t, host = _to_device(a)
-    if t.dtype not in (torch.float32, torch.float64):
-        t = t.to(torch.float64)
+    t, host = float_to_device(a, torch.float64)
     squeeze = t.dim() == 2
     if squeeze:
         t = t[None]
@@ -292,7 +272,7 @@ def nan_gaussian_filter(a, *args, propagate_nan=True, **kwargs):
         result = torch.where(wh_nan, torch.full_like(result, float("nan")), result)
     if squeeze:
         result = result[0]
-    return _to_host(result) if host else result
+    return to_caller(result, host)
 
 
 def growth_markers_multichannel_device(flow: Flow, wvd: torch.Tensor, bt: torch.Tensor, dt_wvd, dt_bt, overlap=0.5,
@@ -326,25 +306,14 @@ def detect_growth_markers_multichannel(flow, wvd, bt, t_sigma=1, overlap=0.5, su
         raise NotImplementedError("subsegment_shrink != 0 (skimage watershed sub-segmentation) is not built here")
     if getattr(wvd, "t", None) is None or getattr(bt, "t", None) is None:
         raise AttributeError("wvd and bt need a time coordinate `.t` (detection.py:216, 219)")
-    on_device = isinstance(wvd, torch.Tensor) and wvd.is_cuda
-    w, _ = _to_device(wvd if isinstance(wvd, torch.Tensor) else _as_numpy(wvd))
-    b, _ = _to_device(bt if isinstance(bt, torch.Tensor) else _as_numpy(bt))
-    if w.dtype not in (torch.float32, torch.float64):
-        w = w.to(torch.float32)
-    if b.dtype not in (torch.float32, torch.float64):
-        b = b.to(torch.float32)
-    r = growth_markers_multichannel_device(flow, w.contiguous(), b.contiguous(), time_diff_minutes(wvd.t),
-                                           time_diff_minutes(bt.t), overlap, min_length, lower_threshold, upper_threshold)
-    if on_device:
+    w, host = float_to_device(wvd, torch.float32)
+    b, _ = float_to_device(bt, torch.float32)
+    r = growth_markers_multichannel_device(flow, w, b, time_diff_minutes(wvd.t), time_diff_minutes(bt.t), overlap,
+                                           min_length, lower_threshold, upper_threshold)
+    if not host:
         return r["wvd_diff_smoothed"], r["bt_diff_smoothed"], r["markers"]
-    out = [_to_host(r["wvd_diff_smoothed"]), _to_host(r["bt_diff_smoothed"]), _to_host(r["markers"])]
-    if hasattr(wvd, "coords") and hasattr(wvd, "dims") and not isinstance(wvd, np.ndarray):
-        try:
-            out = [type(wvd)(out[0], wvd.coords, wvd.dims), type(bt)(out[1], bt.coords, bt.dims),
-                   type(wvd)(out[2], wvd.coords, wvd.dims)]                             # detection.py:249-252
-        except Exception:
-            pass
-    return tuple(out)
+    return (like_input(wvd, to_host(r["wvd_diff_smoothed"])), like_input(bt, to_host(r["bt_diff_smoothed"])),
+            like_input(wvd, to_host(r["markers"])))                                     # detection.py:249-252
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -363,15 +332,14 @@ def combined_edge_field_device(flow: Flow, field: torch.Tensor) -> torch.Tensor:
 
 def get_combined_edge_field(flow: Flow, field, **kwargs):
     """``get_combined_edge_field`` (tobac_flow/detection.py:620-642); numpy in, numpy out."""
-    t, host = _to_device(_as_numpy(field) if not isinstance(field, torch.Tensor) else field)
-    res = combined_edge_field_device(flow, t)
-    return _to_host(res) if host else res
+    t, host = to_device(field)
+    return to_caller(combined_edge_field_device(flow, t), host)
 
 
 def get_watershed_mask(field, erode_distance: int = 1):
     """``get_watershed_mask`` (tobac_flow/detection.py:581-617): ``field <= 0`` or NaN, eroded ``erode_distance`` times with
     the full 3x3x3 structure (border value 1), NaN pixels forced back to True."""
-    t, host = _to_device(_as_numpy(field) if not isinstance(field, torch.Tensor) else field)
+    t, host = to_device(field)
     nan = torch.isnan(t)
     m = ((t <= 0) | nan).to(torch.float32)[None, None]
     for _ in range(int(erode_distance)):

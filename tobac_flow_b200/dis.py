@@ -10,6 +10,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._io import device, stream
 
 PRESET_ULTRAFAST, PRESET_FAST, PRESET_MEDIUM = 0, 1, 2
 
@@ -72,9 +73,8 @@ class DISOpticalFlow:
         tensor in gives a CUDA tensor out.  ``flow`` (an initial flow) is not supported and must be None."""
         if flow is not None:
             raise NotImplementedError("DISOpticalFlow.calc: an initial flow is not supported (pass None)")
-        from .flow import _device, _stream
         on_device = isinstance(I0, torch.Tensor) and I0.is_cuda
-        dev = _device() if not on_device else I0.device
+        dev = device() if not on_device else I0.device
         t0 = I0 if isinstance(I0, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(I0))
         t1 = I1 if isinstance(I1, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(I1))
         if t0.dtype != torch.uint8 or t1.dtype != torch.uint8 or t0.dim() != 2 or tuple(t0.shape) != tuple(t1.shape):
@@ -86,7 +86,7 @@ class DISOpticalFlow:
         ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
         out = torch.empty((2, H, W, 2), dtype=torch.float32, device=dev)
         _lib.check(_lib.load().tf_dis_pairs(t0.data_ptr(), t1.data_ptr(), out[0].data_ptr(), 0, out[1].data_ptr(), 0,
-                                            1, H, W, ctypes.byref(self.params()), ws.data_ptr(), nbytes, _stream()),
+                                            1, H, W, ctypes.byref(self.params()), ws.data_ptr(), nbytes, stream()),
                    "tf_dis_pairs")
         return out[0] if on_device else out[0].cpu().numpy()
 
@@ -94,8 +94,7 @@ class DISOpticalFlow:
 def scale_images(q, model: DISOpticalFlow, scale: int):
     """Stage entry point: scale image ``scale`` of the DIS pyramid of the (n, H, W) uint8 frames ``q`` and its
     spatialGradient -> (img (n, h, w) uint8, gx, gy (n, h, w) int16), numpy."""
-    from .flow import _device, _stream
-    t = torch.from_numpy(np.ascontiguousarray(q, dtype=np.uint8)).to(_device())
+    t = torch.from_numpy(np.ascontiguousarray(q, dtype=np.uint8)).to(device())
     n, H, W = t.shape
     _, _, sizes = model.scale_plan(H, W)
     if scale not in sizes:
@@ -108,5 +107,5 @@ def scale_images(q, model: DISOpticalFlow, scale: int):
     gy = torch.empty((n, h, w), dtype=torch.int16, device=t.device)
     _lib.check(_lib.load().tf_dis_scale_images(t.data_ptr(), n, H, W, ctypes.byref(model.params()), int(scale),
                                                img.data_ptr(), gx.data_ptr(), gy.data_ptr(), ws.data_ptr(), nbytes,
-                                               _stream()), "tf_dis_scale_images")
+                                               stream()), "tf_dis_scale_images")
     return img.cpu().numpy(), gx.cpu().numpy(), gy.cpu().numpy()

@@ -21,6 +21,8 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._io import as_numpy as _as_numpy, device as _device, float_to_device, stream as _stream, to_caller
+from ._io import to_device as _to_device, to_host as _to_host
 from ._lib import NativeError  # noqa: F401  (re-export)
 
 _INTERP = {"nearest": _lib.TF_NEAREST, "linear": _lib.TF_LINEAR, "cubic": _lib.TF_CUBIC, "lanczos": _lib.TF_LANCZOS4}
@@ -37,61 +39,12 @@ def _default_structure():
     return s
 
 
-def _device():
-    if not torch.cuda.is_available():
-        raise NativeError("tobac_flow_b200 needs a CUDA device (there is no CPU fallback)")
-    return torch.device("cuda", torch.cuda.current_device())
-
-
-def _stream():
-    return ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-
-
 def _interp_code(method: str) -> int:
     if method not in _REFERENCE_INTERP_NAMES:
         raise ValueError(f"method must be one of {_REFERENCE_INTERP_NAMES}")  # convolve.py:52-53
     if method not in _INTERP:
         raise NotImplementedError(f"interpolation '{method}' is not built in tobac_flow_b200 (nearest/linear/cubic are)")
     return _INTERP[method]
-
-
-def _as_numpy(data):
-    if isinstance(data, torch.Tensor):
-        return None
-    if hasattr(data, "compute") and hasattr(data, "data") and not isinstance(data, np.ndarray):
-        data = data.compute().data  # xr.DataArray   (flow.py:405-406)
-    elif hasattr(data, "to_numpy"):
-        data = data.to_numpy()      # convolve.py:293-294
-    return np.asarray(data)
-
-
-def _to_device(data, dtype=None):
-    """numpy / DataArray-like / tensor -> contiguous CUDA tensor; returns (tensor, came_from_host)."""
-    dev = _device()
-    if isinstance(data, torch.Tensor):
-        t = data.to(dev)
-        host = not data.is_cuda
-    else:
-        a = np.ascontiguousarray(_as_numpy(data))
-        if a.dtype == np.bool_:
-            a = a.astype(np.int32)
-        t = torch.from_numpy(a).to(dev, non_blocking=False)
-        host = True
-    if dtype is not None and t.dtype != dtype:
-        t = t.to(dtype)
-    return t.contiguous(), host
-
-
-def _to_host(t: torch.Tensor) -> np.ndarray:
-    """Device tensor -> numpy through page-locked memory (torch caches the pinned block, so repeated calls neither
-    page-fault a fresh pageable array nor re-register memory); the array keeps the pinned storage alive."""
-    if not t.is_cuda:
-        return t.numpy()
-    t = t.contiguous()
-    h = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
-    h.copy_(t, non_blocking=True)
-    torch.cuda.current_stream().synchronize()
-    return h.numpy()
 
 
 def _pinned_result_cap() -> int:
@@ -486,7 +439,7 @@ class Flow:
         else:
             res = convolve_device(t, self.forward_flow_device, self.backward_flow_device, structure, method,
                                   fill_value, dtype, reducer)
-        return _to_host(res) if from_host else res
+        return to_caller(res, from_host)
 
     def _convolve_host_pipelined(self, a: np.ndarray, structure, method, fill_value, dtype, reducer, n_taps):
         """Host operand -> host result with the PCIe copies overlapped with the kernels: the operand is uploaded in
@@ -653,10 +606,8 @@ class Flow:
         """``Flow.watershed`` (tobac_flow/flow.py:236-279 -> tobac_flow/watershed.py:17-168): the offset fields are
         prepared on the device, the (value, age) priority flood runs in the native library on the host."""
         from .watershed import watershed
-        return watershed(self.forward_flow_device, self.backward_flow_device, _as_numpy(field) if not isinstance(field, torch.Tensor) else field.cpu().numpy(),
-                         _as_numpy(markers) if not isinstance(markers, torch.Tensor) else markers.cpu().numpy(),
-                         mask=None if mask is None else (_as_numpy(mask) if not isinstance(mask, torch.Tensor) else mask.cpu().numpy()),
-                         connectivity=connectivity)
+        return watershed(self.forward_flow_device, self.backward_flow_device, _as_numpy(field), _as_numpy(markers),
+                         mask=None if mask is None else _as_numpy(mask), connectivity=connectivity)
 
     def label(self, data, structure=None, dtype: type = np.int32, overlap: float = 0, absolute_overlap: int = 1,
               subsegment_shrink: float = 0, peak_min_distance: int = 5):
@@ -868,9 +819,7 @@ def _calculate_flow_tensors(data, model, vr_steps, smoothing_passes, interp_meth
         frames.record_stream(s_in)
         _OPERANDS.put(host_a if host_a.flags.c_contiguous else src.numpy(), frames)   # the operators reuse this copy
     else:
-        frames, _ = _to_device(data)
-        if frames.dtype not in (torch.float32, torch.float64):
-            frames = frames.to(torch.float64)      # integer data: numpy promotes (array - vmin) * factor to float64
+        frames, _ = float_to_device(data, torch.float64)   # integer data: numpy promotes (array - vmin) * factor to float64
     if frames.dim() != 3:
         raise ValueError("data must have shape (t, y, x)")
     frames_b = None
@@ -979,10 +928,8 @@ def smooth_flow_step(forward_flow, backward_flow, method: str = "linear"):
 def pair_to_8bit(frame0, frame1):
     """``to_8bit(linear_norm(stack), 0, 1)`` for one pair (normalisation_utils.py:59-72, 10-33); float64 frames are
     normalised in float64, as numpy does."""
-    a, host = _to_device(np.stack([_as_numpy(frame0), _as_numpy(frame1)]) if not isinstance(frame0, torch.Tensor)
-                         else torch.stack([frame0, frame1]))
-    if a.dtype not in (torch.float32, torch.float64):
-        a = a.to(torch.float64)
+    a, host = float_to_device(np.stack([_as_numpy(frame0), _as_numpy(frame1)]) if not isinstance(frame0, torch.Tensor)
+                              else torch.stack([frame0, frame1]), torch.float64)
     _, H, W = a.shape
     q = torch.empty((2, H, W), dtype=torch.uint8, device=a.device)
     mm = torch.empty((2,), dtype=a.dtype, device=a.device)

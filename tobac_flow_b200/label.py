@@ -14,22 +14,8 @@ import numpy as np
 import torch
 
 from . import _lib
-from .flow import _default_structure, _device, _stream, _to_host, convolve_device
-
-
-def _mask_u8(mask) -> tuple[torch.Tensor, bool]:
-    """Anything array-like -> (T, H, W) uint8 CUDA tensor of ``mask != 0``; second value: input lived on the host."""
-    dev = _device()
-    if isinstance(mask, torch.Tensor):
-        host = not mask.is_cuda
-        t = mask.to(dev)
-    else:
-        a = np.asarray(mask.to_numpy() if hasattr(mask, "to_numpy") else mask)
-        t = torch.from_numpy(np.ascontiguousarray(a != 0)).to(dev)
-        host = True
-    if t.dtype != torch.bool:
-        t = t != 0
-    return t.to(torch.uint8).contiguous(), host
+from ._io import labels_to_device, mask_to_device, stream, to_caller
+from .flow import _default_structure, convolve_device
 
 
 def _connectivity(structure) -> int:
@@ -60,7 +46,7 @@ def flat_label_device(mask_u8: torch.Tensor, connectivity: int = 1) -> tuple[tor
         ws_bytes = int(lib.tf_ccl_workspace_bytes(tc, H, W))
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=mask_u8.device)
         _lib.check(lib.tf_flat_label(mask_u8[done:].data_ptr(), labels[done:].data_ptr(), tc, H, W, connectivity,
-                                     n.data_ptr(), ws.data_ptr(), ws_bytes, _stream()), "tf_flat_label")
+                                     n.data_ptr(), ws.data_ptr(), ws_bytes, stream()), "tf_flat_label")
         if offset:
             part = labels[done:done + tc]
             part += (part > 0).to(torch.int32) * offset
@@ -73,11 +59,9 @@ def flat_label(mask, structure=None, dtype=np.int32):
     """``flat_label`` (tobac_flow/utils/label_utils.py:143-180): per-frame connected components, scipy's numbering."""
     if structure is None:
         structure = _default_structure()
-    m, host = _mask_u8(mask)
+    m, host = mask_to_device(mask)
     labels, _ = flat_label_device(m, _connectivity(structure))
-    if host:
-        return _to_host(labels).astype(dtype, copy=False)
-    return labels
+    return to_caller(labels, host, dtype)
 
 
 def _label_struct(structure):
@@ -106,7 +90,7 @@ def overlap_table_device(flat: torch.Tensor, back: torch.Tensor, fwd: torch.Tens
         counts = torch.empty((cap,), dtype=torch.int32, device=dev)
         _lib.check(lib.tf_label_overlap_count(flat.data_ptr(), back.data_ptr(), fwd.data_ptr(), n, sizes.data_ptr(),
                                               n_labels, keys.data_ptr(), counts.data_ptr(), cap, flags.data_ptr(),
-                                              _stream()), "tf_label_overlap_count")
+                                              stream()), "tf_label_overlap_count")
         fl = flags.cpu()
         if int(fl[1]):
             raise ValueError("flat labels outside 0..max(label)")
@@ -151,7 +135,7 @@ def relabel_device(flat: torch.Tensor, mapping: np.ndarray) -> torch.Tensor:
     if flat.numel():
         map_d = torch.from_numpy(np.ascontiguousarray(mapping, dtype=np.int32)).to(flat.device)
         _lib.check(_lib.load().tf_relabel(flat.data_ptr(), map_d.data_ptr(), out.data_ptr(), flat.numel(),
-                                          len(mapping) - 1, _stream()), "tf_relabel")
+                                          len(mapping) - 1, stream()), "tf_relabel")
     return out
 
 
@@ -165,7 +149,7 @@ def link_overlap_device(flow, flat: torch.Tensor, structure, overlap: float, abs
         return torch.zeros_like(flat), 0
     if n_labels is None:
         mx = torch.zeros((1,), dtype=torch.int32, device=dev)
-        _lib.check(lib.tf_label_max(flat.data_ptr(), n, mx.data_ptr(), _stream()), "tf_label_max")
+        _lib.check(lib.tf_label_max(flat.data_ptr(), n, mx.data_ptr(), stream()), "tf_label_max")
         n_labels = int(mx.item())
         if bool((flat < 0).any()):
             raise ValueError("flat labels must be non-negative")                      # np.bincount raises the same
@@ -184,12 +168,10 @@ def flow_label(flow, mask, structure=None, dtype: type = np.int32, overlap: floa
         raise NotImplementedError("subsegment_shrink != 0 (skimage watershed sub-segmentation) is not built here")
     if tuple(mask.shape) != tuple(flow.shape):
         raise AssertionError("Data input must have the same shape as the Flow object")
-    m, host = _mask_u8(mask)
+    m, host = mask_to_device(mask)
     flat, n_labels = flat_label_device(m, _connectivity(structure))
     out, _ = link_overlap_device(flow, flat, structure, overlap, absolute_overlap, n_labels)
-    if host:
-        return _to_host(out).astype(dtype, copy=False)
-    return out
+    return to_caller(out, host, dtype)
 
 
 def flow_link_overlap(flow, flat_labels, structure=None, dtype: type = np.int32, overlap: float = 0.0,
@@ -199,14 +181,6 @@ def flow_link_overlap(flow, flat_labels, structure=None, dtype: type = np.int32,
         structure = _default_structure()
     if tuple(flat_labels.shape) != tuple(flow.shape):
         raise AssertionError("Data input must have the same shape as the Flow object")
-    dev = _device()
-    if isinstance(flat_labels, torch.Tensor):
-        host = not flat_labels.is_cuda
-        flat = flat_labels.to(dev, torch.int32).contiguous()
-    else:
-        host = True
-        flat = torch.from_numpy(np.ascontiguousarray(np.asarray(flat_labels), dtype=np.int32)).to(dev)
+    flat, host, _ = labels_to_device(flat_labels)
     out, _ = link_overlap_device(flow, flat, structure, overlap, absolute_overlap)
-    if host:
-        return _to_host(out).astype(dtype, copy=False)
-    return out
+    return to_caller(out, host, dtype)

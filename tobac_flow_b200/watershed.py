@@ -19,6 +19,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._io import to_device
 
 
 def _binary_structure(ndim: int, connectivity: int) -> np.ndarray:
@@ -90,10 +91,8 @@ def watershed(forward_flow, backward_flow, field, markers, mask=None, connectivi
             raise ValueError(f"`mask` (shape {mask.shape}) must have same shape as `image` (shape {field.shape})")
     footprint, offset = validate_connectivity(field.ndim, connectivity)
 
-    from .flow import _device
-    dev = _device()        # raises without a CUDA device: there is no CPU path for the device-side preparation
-    to_t = lambda a: (a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a))).to(dev)  # noqa: E731
-    ff, bf = to_t(forward_flow), to_t(backward_flow)
+    # (raises without a CUDA device: there is no CPU path for the device-side preparation)
+    ff, bf = to_device(forward_flow)[0], to_device(backward_flow)[0]
     # np.round = round half to even = torch.round
     rf, rb = torch.round(ff), torch.round(bf)
     pad_offset = offset.copy()
