@@ -56,14 +56,29 @@ typedef enum tf_reducer {
 /* cv2.FarnebackOpticalFlow parameters; tf_fb_default_params() gives the factory defaults that
  * tobac_flow/utils/flow_utils.py:52-53 (cv2.optflow.createOptFlow_Farneback()) uses. */
 typedef struct tf_fb_params {
-    int num_levels;    /* 5   */
-    double pyr_scale;  /* 0.5 (only 0.5 is supported) */
-    int win_size;      /* 13  (odd, <= 25) */
-    int num_iters;     /* 10  */
-    int poly_n;        /* 5   (only 5 is supported) */
+    int num_levels;    /* 5   (0..7) */
+    double pyr_scale;  /* 0.5 (only 0.5 is accepted) */
+    int win_size;      /* 13  (only 13 is accepted) */
+    int num_iters;     /* 10  (>= 1) */
+    int poly_n;        /* 5   (only 5 is accepted) */
     double poly_sigma; /* 1.1 */
     float max_value;   /* clamp applied to the final flow (flow.py:60-61); <= 0 disables */
 } tf_fb_params;
+
+/* cv2.FarnebackOpticalFlow_create(numLevels, pyrScale, fastPyramids = false, winSize, numIters, polyN, polySigma,
+ * flags) over the range that the GPU reproduces: the tf_fb_params fields with wider limits, plus `flags`.
+ * tf_fb_config_default() gives the same factory defaults as tf_fb_default_params(). */
+#define TF_FB_GAUSSIAN 256  /* cv2.OPTFLOW_FARNEBACK_GAUSSIAN: Gaussian instead of box window */
+typedef struct tf_fb_config {
+    int num_levels;    /* 0..15 */
+    double pyr_scale;  /* 0 < pyr_scale < 1 */
+    int win_size;      /* 3..63 with the box window, 4..63 with the Gaussian one (sigma = 0.3 * (win_size / 2)) */
+    int num_iters;     /* >= 1 */
+    int poly_n;        /* 5 or 7 */
+    double poly_sigma; /* > 0 */
+    float max_value;   /* as in tf_fb_params */
+    int flags;         /* 0 or TF_FB_GAUSSIAN (OPTFLOW_USE_INITIAL_FLOW is not supported) */
+} tf_fb_config;
 
 int tf_version(void);
 const char* tf_last_error(void);
@@ -131,6 +146,21 @@ int tf_pair_normalise_u8_f64(const double* f0, const double* f1, long long frame
 int tf_farneback_pairs(const uint8_t* q0, const uint8_t* q1, float* fwd, long long fwd_stride, float* bwd,
                        long long bwd_stride, int n_pairs, int H, int W, const tf_fb_params* p /* host */,
                        void* workspace, size_t workspace_bytes, void* stream);
+
+/* The tf_fb_params entry points above for a tf_fb_config (same schedule, same kernels for the same settings).
+ * Invalid settings fail with TF_ERR_INVALID_ARGUMENT and name the parameter in tf_last_error().
+ * tf_fb_config_level_plan: `hs` / `ws` host arrays of >= 16 ints (may be NULL). */
+void tf_fb_config_default(tf_fb_config* c /* host */);
+int tf_fb_config_level_plan(int H, int W, const tf_fb_config* c /* host */, int* hs /* host */, int* ws /* host */);
+size_t tf_fb_config_workspace_bytes(int n_pairs, int H, int W, const tf_fb_config* c /* host */);
+int tf_farneback_config_pairs(const uint8_t* q0, const uint8_t* q1, float* fwd, long long fwd_stride, float* bwd,
+                              long long bwd_stride, int n_pairs, int H, int W, const tf_fb_config* c /* host */,
+                              void* workspace, size_t workspace_bytes, void* stream);
+int tf_fb_config_pyramid_level(const uint8_t* q0, const uint8_t* q1, int n_pairs, int H, int W,
+                               const tf_fb_config* c /* host */, int level, float* out, void* workspace,
+                               size_t workspace_bytes, int flags, void* stream);
+int tf_fb_config_polyexp(const float* I, int n_img, int h, int w, const tf_fb_config* c /* host */, float* R,
+                         void* stream);
 
 /* cv2.VariationalRefinement parameters; tf_vr_default_params() gives cv2.VariationalRefinement.create()'s defaults
  * (the module-level vr_model of tobac_flow/flow.py:359). */

@@ -2,6 +2,8 @@
 from .flow import (Flow, create_flow, calculate_flow, calculate_flow_2, smooth_flow_step, pair_to_8bit,  # noqa: F401
                    NativeError, operand_cache_clear)
 from .dis import DISOpticalFlow  # noqa: F401
+from .farneback import FarnebackOpticalFlow, OPTFLOW_FARNEBACK_GAUSSIAN  # noqa: F401
 
 __all__ = ["Flow", "create_flow", "calculate_flow", "calculate_flow_2", "smooth_flow_step", "pair_to_8bit",
-           "NativeError", "operand_cache_clear", "DISOpticalFlow"]
+           "NativeError", "operand_cache_clear", "DISOpticalFlow",
+           "FarnebackOpticalFlow", "OPTFLOW_FARNEBACK_GAUSSIAN"]

@@ -28,7 +28,8 @@ EXPORTS = (
     "tf_binary_opening_cross", "tf_grey_opening_cross", "tf_scale_frames", "tf_mask_multiply", "tf_threshold_ge",
     "tf_label_max", "tf_label_overlap_count", "tf_label_link_groups", "tf_relabel", "tf_label_stats",
     "tf_watershed_flood_host", "tf_dis_default_params", "tf_dis_scale_plan", "tf_dis_workspace_bytes", "tf_dis_pairs",
-    "tf_dis_scale_images",
+    "tf_dis_scale_images", "tf_fb_config_default", "tf_fb_config_level_plan", "tf_fb_config_workspace_bytes",
+    "tf_farneback_config_pairs", "tf_fb_config_pyramid_level", "tf_fb_config_polyexp",
 )
 
 KERNEL_CLASSES = ("normalise", "pyramid", "polyexp", "flow_upsample", "fb_iter_coarse", "fb_iter_fullres",
@@ -41,6 +42,10 @@ class FbParams(ctypes.Structure):
         ("num_iters", ctypes.c_int), ("poly_n", ctypes.c_int), ("poly_sigma", ctypes.c_double),
         ("max_value", ctypes.c_float),
     ]
+
+
+class FbConfig(ctypes.Structure):
+    _fields_ = FbParams._fields_ + [("flags", ctypes.c_int)]
 
 
 class VrParams(ctypes.Structure):
@@ -146,6 +151,19 @@ def load():
     lib.tf_dis_pairs.restype = ci
     lib.tf_dis_scale_images.argtypes = [vp, ci, ci, ci, dp, ci, vp, vp, vp, vp, sz, vp]
     lib.tf_dis_scale_images.restype = ci
+    cp = ctypes.POINTER(FbConfig)
+    lib.tf_fb_config_default.argtypes = [cp]
+    lib.tf_fb_config_default.restype = None
+    lib.tf_fb_config_level_plan.argtypes = [ci, ci, cp, ctypes.POINTER(ci), ctypes.POINTER(ci)]
+    lib.tf_fb_config_level_plan.restype = ci
+    lib.tf_fb_config_workspace_bytes.argtypes = [ci, ci, ci, cp]
+    lib.tf_fb_config_workspace_bytes.restype = sz
+    lib.tf_farneback_config_pairs.argtypes = [vp, vp, vp, ll, vp, ll, ci, ci, ci, cp, vp, sz, vp]
+    lib.tf_farneback_config_pairs.restype = ci
+    lib.tf_fb_config_pyramid_level.argtypes = [vp, vp, ci, ci, ci, cp, ci, vp, vp, sz, ci, vp]
+    lib.tf_fb_config_pyramid_level.restype = ci
+    lib.tf_fb_config_polyexp.argtypes = [vp, ci, ci, ci, cp, vp, vp]
+    lib.tf_fb_config_polyexp.restype = ci
     lib.tf_profile_enable.argtypes = [ci]
     lib.tf_profile_read.argtypes = [ci, ctypes.POINTER(cd), ctypes.POINTER(cd), ctypes.POINTER(ll)]
     for name in ("tf_profile_enable", "tf_profile_reset", "tf_profile_read", "tf_fb_level_plan", "tf_fb_poly_constants", "tf_pair_normalise_u8", "tf_farneback_pairs",

@@ -10,14 +10,24 @@ struct BlurTaps {
     float w[kMaxBlurTaps];
 };
 
+// Levels of a frame at most 5424 px on its short side need up to 421 taps (one level at pyr_scale 32 / 5424);
+// blurs wider than kMaxBlurTaps take the two-pass kernels with these taps.
+constexpr int kMaxWideBlurTaps = 511;
+struct WideBlurTaps {
+    int ksize;
+    float w[kMaxWideBlurTaps];
+};
+
 struct PolyConsts {
-    float g[6], xg[6], xxg[6];  // g[k], k = 0..5 (symmetric / antisymmetric about 0)
+    int n;                      // poly_n: 5 or 7
+    float g[8], xg[8], xxg[8];  // g[k], k = 0..n (symmetric / antisymmetric about 0)
     float ig11, ig03, ig33, ig55;
 };
 PolyConsts make_poly_consts(int n, double sigma);
 
 // level image for 2*n_pairs images: out (2*n_pairs, h, w); tmp >= 2*n_pairs * rows*W floats
 // two_pass: the separable path through `tmp` instead of the fused tile kernels (same bits; kept for parity tests)
+// ksize > kMaxBlurTaps: the two-pass path with WideBlurTaps (two_pass is then implied)
 int launch_pyramid_level(const uint8_t* q0, const uint8_t* q1, int n_pairs, int H, int W, int h, int w, int ksize,
                          double sigma, float* tmp, float* out, cudaStream_t s, bool two_pass = false);
 
@@ -55,5 +65,11 @@ bool fb_iteration_can_fuse_upsample();
 int launch_fb_iteration(const float* R, long long img_stride, const float* flow_in, float* out_fwd, long long fwd_stride, float* out_bwd,
                         long long bwd_stride, int n_pairs, int h, int w, int win, float clamp, bool full_res, cudaStream_t s,
                         const UpArgs* up = nullptr);
+
+// The same Jacobi iteration for any window: box (win_size 3..63) or, with `gaussian`, OpenCV's Gaussian window
+// (win_size 4..63).  Same buffers and addressing as launch_fb_iteration, no fused up-sampling.
+int launch_fb_iteration_general(const float* R, long long img_stride, const float* flow_in, float* out_fwd,
+                                long long fwd_stride, float* out_bwd, long long bwd_stride, int n_pairs, int h, int w,
+                                int win, bool gaussian, float clamp, bool full_res, cudaStream_t s);
 
 }  // namespace tf

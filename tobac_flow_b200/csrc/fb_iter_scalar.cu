@@ -12,22 +12,6 @@
 
 namespace tf {
 
-__device__ __forceinline__ float4 ld_stream(const float4* p) {
-    float4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-    return r;
-}
-__device__ __forceinline__ float2 ld_stream(const float2* p) {
-    float2 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v2.f32 {%0, %1}, [%2];" : "=f"(r.x), "=f"(r.y) : "l"(p));
-    return r;
-}
-__device__ __forceinline__ float ld_stream1(const float* p) {
-    float r;
-    asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(r) : "l"(p));
-    return r;
-}
-
 template <bool TM>
 struct ScalarCfg {
     static constexpr int NT = 128, HK = 4, OUT_W = NT - 2 * IT_HALO;
@@ -37,75 +21,6 @@ struct ScalarCfg {
     static constexpr int VBUF_FLOATS = 8 * 5 * NT;           // 2 buffers x 4 rows of vertical sums
     static constexpr int SMEM_BYTES = (RING_FLOATS + VBUF_FLOATS) * (int)sizeof(float);
 };
-
-// Everything one pixel's FarnebackUpdateMatrices reads: R0 at the pixel, the four bilinear taps of R1 at p + flow.
-struct Taps {
-    float4 c;  float c4;                 // R0: (c0..c3), c4
-    float4 p00, p01, p10, p11;           // R1 float4 plane taps
-    float q00, q01, q10, q11;            // R1 c4 plane taps
-    float fx, fy, dx, dy;                // bilinear fractions and the flow
-    int y;                               // image row (replicate-clamped)
-    bool inside;
-};
-
-struct RPlanes {
-    const float4* R0a; const float* R0b; const float4* R1a; const float* R1b;
-};
-
-// issue the loads of one pixel (addresses are always valid; `inside` says whether the R1 taps are used)
-__device__ __forceinline__ void issue_taps(Taps& t, const RPlanes& R, int w, int h, int x, int y, float2 f) {
-    const int o = y * w + x;
-    t.y = y;
-    t.dx = f.x;
-    t.dy = f.y;
-    const float fx = __fadd_rn((float)x, f.x), fy = __fadd_rn((float)y, f.y);
-    const float flx = floorf(fx), fly = floorf(fy);
-    const int x1 = (int)flx, y1 = (int)fly;
-    t.fx = __fsub_rn(fx, flx);
-    t.fy = __fsub_rn(fy, fly);
-    t.inside = (unsigned)x1 < (unsigned)(w - 1) && (unsigned)y1 < (unsigned)(h - 1);
-    // out-of-image positions read a clamped (valid) 2x2 footprint whose values are then ignored
-    const int xc = max(min(x1, w - 2), 0), yc = max(min(y1, h - 2), 0);
-    const float4* a0 = R.R1a + (yc * w + xc);
-    const float4* a1 = a0 + w;
-    const float* b0 = R.R1b + (yc * w + xc);
-    const float* b1 = b0 + w;
-    t.c = ld_stream(R.R0a + o);      // touched once by this CTA: do not displace the gather footprint in L1
-    t.c4 = ld_stream1(R.R0b + o);
-    t.p00 = __ldg(a0);
-    t.p01 = __ldg(a0 + 1);
-    t.p10 = __ldg(a1);
-    t.p11 = __ldg(a1 + 1);
-    t.q00 = __ldg(b0);
-    t.q01 = __ldg(b0 + 1);
-    t.q10 = __ldg(b1);
-    t.q11 = __ldg(b1 + 1);
-}
-
-// FarnebackUpdateMatrices for one pixel from its loaded taps (explicit roundings: see fb_iter_common.cuh)
-__device__ __forceinline__ void matrix_from_taps(const Taps& t, int h, float sc_x, bool band_x, float m[5]) {
-    float r2, r3, r4, r5, r6;
-    if (t.inside) {
-        float a00, a01, a10, a11;
-        bilinear_weights(t.fx, t.fy, a00, a01, a10, a11);
-        r2 = blend4(a00, a01, a10, a11, t.p00.x, t.p01.x, t.p10.x, t.p11.x);
-        r3 = blend4(a00, a01, a10, a11, t.p00.y, t.p01.y, t.p10.y, t.p11.y);
-        r4 = blend4(a00, a01, a10, a11, t.p00.z, t.p01.z, t.p10.z, t.p11.z);
-        r5 = blend4(a00, a01, a10, a11, t.p00.w, t.p01.w, t.p10.w, t.p11.w);
-        r6 = blend4(a00, a01, a10, a11, t.q00, t.q01, t.q10, t.q11);
-        r4 = __fmul_rn(__fadd_rn(t.c.z, r4), 0.5f);
-        r5 = __fmul_rn(__fadd_rn(t.c.w, r5), 0.5f);
-        r6 = __fmul_rn(__fadd_rn(t.c4, r6), 0.25f);
-    } else {
-        r2 = r3 = 0.f;
-        r4 = t.c.z;
-        r5 = t.c.w;
-        r6 = __fmul_rn(t.c4, 0.5f);
-    }
-    r2 = __fmul_rn(__fsub_rn(t.c.x, r2), 0.5f);
-    r3 = __fmul_rn(__fsub_rn(t.c.y, r3), 0.5f);
-    terms_from_blend(r2, r3, r4, r5, r6, t.dx, t.dy, border_scale(sc_x, band_x, t.y, h), m);
-}
 
 template <bool TM>
 __global__ void __launch_bounds__(128, 4)

@@ -1,23 +1,32 @@
-// K3: Farneback polynomial expansion (OpenCV FarnebackPolyExp, polyN = 5): separable 11-tap tile convolution with
-// replicate borders.  Input level image I (h, w) fp32 -> per image a float4 plane (c0..c3) followed by a float plane
+// K3: Farneback polynomial expansion (OpenCV FarnebackPolyExp, polyN = 5 or 7): separable (2N+1)-tap tile convolution
+// with replicate borders.  Input level image I (h, w) fp32 -> per image a float4 plane (c0..c3) followed by a float plane
 // (c4), so the iteration kernel's bilinear gathers are one 16-byte and one 4-byte coalesced load per tap.
-// Shared-memory tile with a 5-pixel halo; both passes are register-blocked (vertical: a 26-row column window per
-// thread for 16 outputs; horizontal: 16 values of each moment row per thread for 4 outputs).
+// Shared-memory tile with an N-pixel halo; both passes are register-blocked (vertical: a (16 + 2N)-row column window per
+// thread for 16 outputs; horizontal: 4 + 2N values of each moment row per thread for 4 outputs).
 // HBM traffic: 4 B/px read (+ halo re-reads that hit L2) and 20 B/px written.
 #include "farneback_internal.cuh"
 
 namespace tf {
 
-constexpr int PE_N = 5;
-constexpr int PE_SW = 128;                    // region columns incl. halo (also the shared-memory pitch)
-constexpr int PE_TW = PE_SW - 2 * PE_N;       // 118 output columns per tile
-constexpr int PE_TH = 32;                     // output rows per tile
-constexpr int PE_SH = PE_TH + 2 * PE_N;       // 42 rows incl. halo
-constexpr int PE_VSEG = 16;                   // rows per thread in the vertical pass
-constexpr int PE_SMEM_BYTES = (PE_SH * PE_SW + 3 * PE_TH * PE_SW + 4) * (int)sizeof(float);  // +4: the last group's 16-value load overhangs
+template <int N>
+struct PeCfg {
+    static constexpr int SW = 128;                 // region columns incl. halo (also the shared-memory pitch)
+    static constexpr int TW = SW - 2 * N;          // output columns per tile
+    static constexpr int TH = 32;                  // output rows per tile
+    static constexpr int SH = TH + 2 * N;          // rows incl. halo
+    static constexpr int VSEG = 16;                // rows per thread in the vertical pass
+    static constexpr int NV = (4 + 2 * N + 3) / 4; // float4 loads of a moment row per thread in the horizontal pass
+    static constexpr int GROUPS = (TW + 3) / 4;    // groups of 4 output columns (the last one may overhang TW)
+    // +4: the last group's loads overhang
+    static constexpr int SMEM_BYTES = (SH * SW + 3 * TH * SW + 4) * (int)sizeof(float);
+    static_assert(4 * (GROUPS - 1) + 4 * NV <= SW + 4, "horizontal loads stay inside the tile + pad");
+};
 
+template <int N>
 __global__ void __launch_bounds__(256) polyexp_kernel(const float* __restrict__ I, float* __restrict__ R,
                                                       long long img_stride, int h, int w, PolyConsts pc) {
+    using C = PeCfg<N>;
+    constexpr int PE_N = N, PE_SW = C::SW, PE_TW = C::TW, PE_TH = C::TH, PE_SH = C::SH, PE_VSEG = C::VSEG;
     extern __shared__ __align__(16) float pe_smem[];
     float (*s_in)[PE_SW] = reinterpret_cast<float (*)[PE_SW]>(pe_smem);
     float (*s_v)[PE_TH][PE_SW] = reinterpret_cast<float (*)[PE_TH][PE_SW]>(pe_smem + PE_SH * PE_SW);
@@ -26,8 +35,8 @@ __global__ void __launch_bounds__(256) polyexp_kernel(const float* __restrict__ 
     const float* src = I + (long long)img * h * w;
     const int tid = threadIdx.x;
 
-    // tile + 5-px halo, replicate-clamped (the clamp IS OpenCV's border rule for both passes)
-    // (all 21 loads of a thread are issued before the first shared-memory store: one memory round trip, not 21)
+    // tile + N-px halo, replicate-clamped (the clamp IS OpenCV's border rule for both passes)
+    // (all loads of a thread are issued before the first shared-memory store: one memory round trip, not one per load)
     {
         static_assert((PE_SH * PE_SW) % 256 == 0 && PE_SW == 128, "tile load: 2 rows per pass of the 256 threads");
         constexpr int PASSES = PE_SH * PE_SW / 256;
@@ -73,16 +82,16 @@ __global__ void __launch_bounds__(256) polyexp_kernel(const float* __restrict__ 
     const int plane = h * w;
     float4* dst_a = reinterpret_cast<float4*>(R + (long long)img * img_stride);
     float* dst_b = R + (long long)img * img_stride + 4 * (long long)plane;
-    constexpr int GROUPS = PE_SW / 4 - 2;     // 30 groups of 4 output columns (the last one is partly beyond PE_TW)
+    constexpr int GROUPS = C::GROUPS, NV = C::NV;
     const bool wide_ok = (w & 1) == 0 && (reinterpret_cast<uintptr_t>(dst_a) & 31) == 0;   // 32-byte aligned texel pairs
     for (int task = tid; task < PE_TH * GROUPS; task += 256) {
         const int r = task / GROUPS, cgp = task - r * GROUPS;
         const int c0 = 4 * cgp;               // first output column (tile-relative); its region column is c0 + PE_N
         const int gy = y0 + r;
         if (gy >= h || x0 + c0 >= w) continue;
-        float v0[16], v1[16], v2[16];         // region columns c0 .. c0+15  (outputs need c0 .. c0+13)
+        float v0[4 * NV], v1[4 * NV], v2[4 * NV];   // region columns c0 .. c0+4NV-1  (outputs need c0 .. c0+3+2N)
 #pragma unroll
-        for (int q = 0; q < 4; ++q) {
+        for (int q = 0; q < NV; ++q) {
             const float4 a = *reinterpret_cast<const float4*>(&s_v[0][r][c0 + 4 * q]);
             const float4 b = *reinterpret_cast<const float4*>(&s_v[1][r][c0 + 4 * q]);
             const float4 d = *reinterpret_cast<const float4*>(&s_v[2][r][c0 + 4 * q]);
@@ -143,25 +152,35 @@ __global__ void __launch_bounds__(256) polyexp_kernel(const float* __restrict__ 
     }
 }
 
-int launch_polyexp(const float* I, float* R, long long img_stride, int n_img, int h, int w, const PolyConsts& pc,
-                   cudaStream_t s) {
+template <int N>
+static void launch_polyexp_n(const float* I, float* R, long long img_stride, int n_img, int h, int w, const PolyConsts& pc,
+                             cudaStream_t s) {
+    using C = PeCfg<N>;
     // (the attribute is per device: set it on every call, it is cheap)
-    cudaFuncSetAttribute(polyexp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PE_SMEM_BYTES);
-    LaunchTimer lt(KC_POLYEXP, 24.0 * h * w * n_img, s, cdiv(n_img, 65535));
+    cudaFuncSetAttribute(polyexp_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
     for (int z0 = 0; z0 < n_img; z0 += 65535) {
         const int nz = min(n_img - z0, 65535);
-        dim3 g(cdiv(w, PE_TW), cdiv(h, PE_TH), nz);
-        polyexp_kernel<<<g, 256, PE_SMEM_BYTES, s>>>(I + (long long)z0 * h * w, R + (long long)z0 * img_stride, img_stride, h,
-                                                     w, pc);
+        dim3 g(cdiv(w, C::TW), cdiv(h, C::TH), nz);
+        polyexp_kernel<N><<<g, 256, C::SMEM_BYTES, s>>>(I + (long long)z0 * h * w, R + (long long)z0 * img_stride,
+                                                        img_stride, h, w, pc);
     }
+}
+
+int launch_polyexp(const float* I, float* R, long long img_stride, int n_img, int h, int w, const PolyConsts& pc,
+                   cudaStream_t s) {
+    if (pc.n != 5 && pc.n != 7) { set_error("polyexp: poly_n %d is not built (5 or 7)", pc.n); return TF_ERR_UNSUPPORTED; }
+    LaunchTimer lt(KC_POLYEXP, 24.0 * h * w * n_img, s, cdiv(n_img, 65535));
+    if (pc.n == 5) launch_polyexp_n<5>(I, R, img_stride, n_img, h, w, pc, s);
+    else launch_polyexp_n<7>(I, R, img_stride, n_img, h, w, pc, s);
     return check_launch("polyexp");
 }
 
 // FarnebackPrepareGaussian: fp32 taps, fp64 moment matrix inverse (closed form for the sparse 6x6)
 PolyConsts make_poly_consts(int n, double sigma) {
     PolyConsts pc{};
+    pc.n = n;
     if (sigma < 1.1920929e-07) sigma = n * 0.3;
-    float g[11];
+    float g[15];
     double s = 0;
     for (int x = -n; x <= n; ++x) {
         g[x + n] = (float)exp(-x * x / (2 * sigma * sigma));

@@ -35,9 +35,11 @@ __device__ __forceinline__ void resize_coord(int d, double scale, int src_n, int
 }
 
 // pass A.  tmp: (n_img, h*rp, W) fp32, rp = rows per destination row (1 when h == H, else 2)
+// (Taps: BlurTaps, or WideBlurTaps for the blurs wider than kMaxBlurTaps)
+template <class Taps>
 __global__ void __launch_bounds__(256) blur_v_kernel(const uint8_t* __restrict__ q0, const uint8_t* __restrict__ q1,
                                                      float* __restrict__ tmp, int H, int W, int h, int rp,
-                                                     double scale_y, BlurTaps taps) {
+                                                     double scale_y, Taps taps) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
     const int r = blockIdx.y;
     const int img = blockIdx.z;  // 2*pair + which
@@ -605,9 +607,10 @@ __global__ void __launch_bounds__(256) blur_h4_fullres_kernel(const float* __res
 }
 
 // pass B.  out: (n_img, h, w) fp32
+template <class Taps>
 __global__ void __launch_bounds__(256) blur_h_resize_kernel(const float* __restrict__ tmp, float* __restrict__ out, int W,
                                                             int h, int w, int rp, double scale_x, double scale_y,
-                                                            int H, BlurTaps taps) {
+                                                            int H, Taps taps) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const int j = blockIdx.y;
     const int img = blockIdx.z;
@@ -717,16 +720,15 @@ __global__ void __launch_bounds__(256) flow_upsample_kernel(const float2* __rest
     }
 }
 
-int launch_pyramid_level(const uint8_t* q0, const uint8_t* q1, int n_pairs, int H, int W, int h, int w, int ksize,
-                         double sigma, float* tmp, float* out, cudaStream_t s, bool two_pass) {
-    BlurTaps taps;
+// cv::getGaussianKernel(ksize, sigma, CV_32F)
+template <class Taps>
+static void gaussian_taps(Taps& taps, int ksize, double sigma) {
     taps.ksize = ksize;
-    if (ksize > kMaxBlurTaps) { set_error("pyramid: blur kernel too wide (%d)", ksize); return TF_ERR_UNSUPPORTED; }
     if (sigma <= 0 && ksize == 3) {
         taps.w[0] = 0.25f; taps.w[1] = 0.5f; taps.w[2] = 0.25f;
     } else {
         if (sigma <= 0) sigma = 0.3 * ((ksize - 1) * 0.5 - 1) + 0.8;
-        double sum = 0, v[kMaxBlurTaps];
+        double sum = 0, v[sizeof(taps.w) / sizeof(float)];
         for (int i = 0; i < ksize; ++i) {
             double x = i - (ksize - 1) * 0.5;
             v[i] = exp(-0.5 * x * x / (sigma * sigma));
@@ -734,6 +736,38 @@ int launch_pyramid_level(const uint8_t* q0, const uint8_t* q1, int n_pairs, int 
         }
         for (int i = 0; i < ksize; ++i) taps.w[i] = (float)(v[i] / sum);
     }
+}
+
+// A level whose blur is wider than kMaxBlurTaps (deep levels, small pyr_scale): the separable two-pass kernels with the
+// taps in a larger parameter block.  Such levels are small (at most 1/20 of the frame per side), so the ksize
+// multiply-adds per pixel and pass cost little next to the full-resolution level.
+static int launch_pyramid_level_wide(const uint8_t* q0, const uint8_t* q1, int n_pairs, int H, int W, int h, int w,
+                                     int ksize, double sigma, float* tmp, float* out, cudaStream_t s) {
+    if (ksize > kMaxWideBlurTaps) { set_error("pyramid: blur kernel too wide (%d)", ksize); return TF_ERR_UNSUPPORTED; }
+    WideBlurTaps taps;
+    gaussian_taps(taps, ksize, sigma);
+    const int rp = (h == H) ? 1 : 2;
+    const double sx = (double)W / w, sy = (double)H / h;
+    const int n_img = 2 * n_pairs;
+    LaunchTimer lt(KC_PYRAMID, (2.0 * H * W + 8.0 * h * w) * n_pairs, s, 2 * cdiv(n_img, 65534));
+    for (int z0 = 0; z0 < n_img; z0 += 65534) {
+        const int nz = min(n_img - z0, 65534);
+        const uint8_t* a0 = q0 + (long long)(z0 / 2) * H * W;
+        const uint8_t* a1 = q1 + (long long)(z0 / 2) * H * W;
+        float* tz = tmp + (long long)z0 * h * rp * W;
+        dim3 ga(cdiv(W, 256), h * rp, nz);
+        blur_v_kernel<<<ga, 256, 0, s>>>(a0, a1, tz, H, W, h, rp, sy, taps);
+        dim3 gb(cdiv(w, 256), h, nz);
+        blur_h_resize_kernel<<<gb, 256, 0, s>>>(tz, out + (long long)z0 * h * w, W, h, w, rp, sx, sy, H, taps);
+    }
+    return check_launch("pyramid level (wide blur)");
+}
+
+int launch_pyramid_level(const uint8_t* q0, const uint8_t* q1, int n_pairs, int H, int W, int h, int w, int ksize,
+                         double sigma, float* tmp, float* out, cudaStream_t s, bool two_pass) {
+    if (ksize > kMaxBlurTaps) return launch_pyramid_level_wide(q0, q1, n_pairs, H, W, h, w, ksize, sigma, tmp, out, s);
+    BlurTaps taps;
+    gaussian_taps(taps, ksize, sigma);
     const int rp = (h == H) ? 1 : 2;
     const double sx = (double)W / w, sy = (double)H / h;
     const int n_img = 2 * n_pairs;

@@ -26,7 +26,7 @@ inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // host-side cvRound (round half to even)
 inline int cv_round(double v) { return (int)nearbyint(v); }
 
-constexpr int kMaxLevels = 8;
+constexpr int kMaxLevels = 16;
 
 struct LevelPlan {
     int n;                 // number of levels processed (coarsest first)
@@ -34,7 +34,7 @@ struct LevelPlan {
     double sigma[kMaxLevels];
 };
 
-LevelPlan make_level_plan(int H, int W, const tf_fb_params& p);
+LevelPlan make_level_plan(int H, int W, const tf_fb_config& c);
 
 // kernel classes for launch accounting (tf_profile_*)
 enum KClass {

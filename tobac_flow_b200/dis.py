@@ -68,6 +68,10 @@ class DISOpticalFlow:
         self.scale_plan(H, W)      # raises for a frame OpenCV refuses
         return int(_lib.load().tf_dis_workspace_bytes(n_pairs, H, W, ctypes.byref(self._p)))
 
+    def _run_pairs(self, q0, q1, fwd, fwd_stride, bwd, bwd_stride, n_pairs, H, W, params, ws, ws_bytes, st):
+        _lib.check(_lib.load().tf_dis_pairs(q0, q1, fwd, fwd_stride, bwd, bwd_stride, n_pairs, H, W, ctypes.byref(params),
+                                            ws, ws_bytes, st), "tf_dis_pairs")
+
     def calc(self, I0, I1, flow=None):
         """Flow from ``I0`` to ``I1`` ((H, W) uint8 each) as (H, W, 2) float32: numpy in gives numpy out, a CUDA
         tensor in gives a CUDA tensor out.  ``flow`` (an initial flow) is not supported and must be None."""
@@ -85,9 +89,8 @@ class DISOpticalFlow:
         nbytes = self.workspace_bytes(1, H, W)
         ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
         out = torch.empty((2, H, W, 2), dtype=torch.float32, device=dev)
-        _lib.check(_lib.load().tf_dis_pairs(t0.data_ptr(), t1.data_ptr(), out[0].data_ptr(), 0, out[1].data_ptr(), 0,
-                                            1, H, W, ctypes.byref(self.params()), ws.data_ptr(), nbytes, stream()),
-                   "tf_dis_pairs")
+        self._run_pairs(t0.data_ptr(), t1.data_ptr(), out[0].data_ptr(), 0, out[1].data_ptr(), 0, 1, H, W,
+                        self.params(), ws.data_ptr(), nbytes, stream())
         return out[0] if on_device else out[0].cpu().numpy()
 
 

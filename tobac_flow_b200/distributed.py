@@ -31,9 +31,10 @@ def shard_bounds(T: int, world: int, rank: int):
 class CudaOps:
     """The product back-end: the CUDA kernels through the C ABI."""
 
-    def calculate_flow(self, frames, fwd, bwd, smoothing_passes, interp_method, max_value, vr_steps=0):
+    def calculate_flow(self, frames, fwd, bwd, smoothing_passes, interp_method, max_value, vr_steps=0, model=None):
         from .flow import calculate_flow_device
-        calculate_flow_device(frames, fwd, bwd, smoothing_passes, interp_method, max_value, vr_steps=vr_steps)
+        calculate_flow_device(frames, fwd, bwd, smoothing_passes, interp_method, max_value, vr_steps=vr_steps,
+                              model=model)
 
     def finalise(self, fwd, bwd, max_value, clamp_all, mirror_first, mirror_last):
         from .flow import finalise_flow_device
@@ -235,8 +236,9 @@ class ShardedFlow:
 
 
 def create_flow_sharded(shard: Shard, smoothing_passes=0, interp_method="linear", max_value=20, ops=None, group=None,
-                        exchange=True, fwd=None, bwd=None, vr_steps=0) -> ShardedFlow:
-    """``create_flow`` for one rank of a time-sharded series; ``shard.buf[1:-1]`` holds the rank's frames."""
+                        exchange=True, fwd=None, bwd=None, vr_steps=0, model=None) -> ShardedFlow:
+    """``create_flow`` for one rank of a time-sharded series; ``shard.buf[1:-1]`` holds the rank's frames.
+    ``model``: as for ``create_flow`` (None is "Farneback")."""
     ops = ops or CudaOps()
     rank, world = shard.rank, shard.world
     T_loc, H, W = shard.local.shape
@@ -250,6 +252,10 @@ def create_flow_sharded(shard: Shard, smoothing_passes=0, interp_method="linear"
         assert fwd.dtype == torch.float32 and bwd.dtype == torch.float32 and fwd.is_contiguous() and bwd.is_contiguous()
         assert tuple(fwd.shape) == (T_loc, H, W, 2) and tuple(bwd.shape) == (T_loc + 1, H, W, 2), "fwd (T_loc,..) / bwd (T_loc+1,..)"
     kw = dict(vr_steps=vr_steps) if vr_steps else {}
+    if model is not None:        # (passed only when given: a back-end may have no `model` parameter)
+        from .flow import _check_model
+        _check_model(model, vr_steps)
+        kw["model"] = model
     halo_ready = None
     if exchange and world > 1 and dev.type == "cuda":
         # the one-frame halos travel on a side stream (NCCL p2p over NVLink) while the interior pairs, which only read

@@ -645,14 +645,16 @@ except Exception:  # pragma: no cover
 # ------------------------------------------------------------------------------------------------------------------
 # flow construction
 # ------------------------------------------------------------------------------------------------------------------
-def _is_dis(model) -> bool:
+def _is_model_object(model) -> bool:
     from .dis import DISOpticalFlow
-    return isinstance(model, DISOpticalFlow)
+    from .farneback import FarnebackOpticalFlow
+    return isinstance(model, (DISOpticalFlow, FarnebackOpticalFlow))
 
 
 def _check_model(model, vr_steps: int):
-    """``model``: the reference's model name, or a :class:`tobac_flow_b200.DISOpticalFlow` instance."""
-    if _is_dis(model):
+    """``model``: the reference's model name, or a :class:`tobac_flow_b200.FarnebackOpticalFlow` or
+    :class:`tobac_flow_b200.DISOpticalFlow` instance."""
+    if _is_model_object(model):
         return
     if model not in _REFERENCE_MODELS:
         raise ValueError(  # utils/flow_utils.py:72-75
@@ -670,12 +672,12 @@ def _pair_batch(n_pairs: int, H: int, W: int, params, vr: bool = False, model=No
     # (the answer for a shape is remembered: `cudaMemGetInfo` is a driver call that can wait milliseconds behind a
     # monitoring query -- nvidia-smi -- and it sits in front of a call's first kernel launch; a shape whose workspace
     # allocation fails later drops its entry, see calculate_flow_device)
-    dis = _is_dis(model)
-    key = (torch.cuda.current_device(), n_pairs, H, W, bool(vr), model.key() if dis else params.num_levels,
+    obj = _is_model_object(model)
+    key = (torch.cuda.current_device(), n_pairs, H, W, bool(vr), model.key() if obj else params.num_levels,
            os.environ.get("TF_PAIR_BATCH_MPX"))
     if key in _PAIR_BATCH_CACHE:
         return _PAIR_BATCH_CACHE[key]
-    per_pair = (model.workspace_bytes(1, H, W) if dis else _lib.workspace_bytes(1, H, W, params)) + 2 * H * W
+    per_pair = (model.workspace_bytes(1, H, W) if obj else _lib.workspace_bytes(1, H, W, params)) + 2 * H * W
     if vr:
         per_pair += int(_lib.load().tf_vr_workspace_bytes(1, H, W))
     free, _ = torch.cuda.mem_get_info()
@@ -701,7 +703,8 @@ def calculate_flow_device(frames: torch.Tensor, fwd: torch.Tensor, bwd: torch.Te
     ``frames`` (T, H, W) float32 or float64; ``fwd``/``bwd`` (>= T, H, W, 2) float32.  With ``next_frames`` the pairs are
     (frames[i], next_frames[i]) and results go to fwd[i], bwd[i + 1] for every i (``calculate_flow_2``).
     ``max_value`` fuses the clamp of ``create_flow`` into the last kernel when no smoothing follows.
-    ``model``: None (Farneback) or a :class:`tobac_flow_b200.DISOpticalFlow`.
+    ``model``: None or "Farneback" (OpenCV's factory Farneback), or a :class:`tobac_flow_b200.FarnebackOpticalFlow` or
+    :class:`tobac_flow_b200.DISOpticalFlow`.
     """
     lib = _lib.load()
     T, H, W = frames.shape
@@ -711,10 +714,10 @@ def calculate_flow_device(frames: torch.Tensor, fwd: torch.Tensor, bwd: torch.Te
     interp = _interp_code(interp_method)
     use_vr = bool(vr_steps) and vr_steps > 0   # flow.py:513-519: one refinement whenever vr_steps > 0
     fuse_clamp = (max_value is not None) and smoothing_passes == 0 and not use_vr
-    dis = _is_dis(model)
+    obj = _is_model_object(model)
     params = _lib.default_params(max_value if fuse_clamp else 0.0)
-    if dis:
-        dis_params = model.params(max_value if fuse_clamp else 0.0)
+    if obj:
+        model_params = model.params(max_value if fuse_clamp else 0.0)
     nb = batch or _pair_batch(n_pairs, H, W, params, use_vr, model)
     if batch_plan is None:
         batch_plan = [min(nb, n_pairs - p0) for p0 in range(0, n_pairs, nb)]
@@ -727,7 +730,7 @@ def calculate_flow_device(frames: torch.Tensor, fwd: torch.Tensor, bwd: torch.Te
     f64 = frames.dtype == torch.float64        # float64 frames are normalised in float64, as numpy does for the reference
     mm = torch.empty((2 * nb,), dtype=frames.dtype, device=dev)
     normalise = lib.tf_pair_normalise_u8_f64 if f64 else lib.tf_pair_normalise_u8
-    ws_bytes = model.workspace_bytes(nb, H, W) if dis else _lib.workspace_bytes(nb, H, W, params)
+    ws_bytes = model.workspace_bytes(nb, H, W) if obj else _lib.workspace_bytes(nb, H, W, params)
     try:
         ws = torch.empty((ws_bytes,), dtype=torch.uint8, device=dev)
     except torch.cuda.OutOfMemoryError:
@@ -756,9 +759,9 @@ def calculate_flow_device(frames: torch.Tensor, fwd: torch.Tensor, bwd: torch.Te
                    "tf_pair_normalise_u8")
         fo = fwd.data_ptr() + p0 * hw * 2 * 4
         bo = bwd.data_ptr() + (p0 + 1) * hw * 2 * 4
-        if dis:
-            _lib.check(lib.tf_dis_pairs(q0.data_ptr(), q1.data_ptr(), fo, hw * 2, bo, hw * 2, n, H, W,
-                                        ctypes.byref(dis_params), ws.data_ptr(), ws_bytes, st), "tf_dis_pairs")
+        if obj:
+            model._run_pairs(q0.data_ptr(), q1.data_ptr(), fo, hw * 2, bo, hw * 2, n, H, W, model_params, ws.data_ptr(),
+                             ws_bytes, st)
         else:
             _lib.check(lib.tf_farneback_pairs(q0.data_ptr(), q1.data_ptr(), fo, hw * 2, bo, hw * 2, n, H, W,
                                               ctypes.byref(params), ws.data_ptr(), ws_bytes, st), "tf_farneback_pairs")
@@ -901,8 +904,8 @@ def create_flow(data, model: str = "Farneback", vr_steps: int = 0, smoothing_pas
                 interp_method: str = "linear", max_value=20) -> Flow:
     """``create_flow`` (tobac_flow/flow.py:23-65): flow vectors for ``data`` (t, y, x), clamped to +-max_value.
 
-    ``model`` is "Farneback" or a :class:`tobac_flow_b200.DISOpticalFlow` (as for ``calculate_flow`` /
-    ``calculate_flow_2``).
+    ``model`` is "Farneback" or a :class:`tobac_flow_b200.FarnebackOpticalFlow` or
+    :class:`tobac_flow_b200.DISOpticalFlow` instance (as for ``calculate_flow`` / ``calculate_flow_2``).
 
     The returned ``Flow`` keeps the vectors on the GPU.
     """
